@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — boosting iterations/second of the GBT histogram split finder (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2] [--dump-outputs DIR]
 
 A "step" is one boosting iteration (one tree) over the resident synthetic matrix.  Default workload
 is BASELINE.json's headline configuration C3: 10M rows x 200 numerical features, 256 bins,
@@ -503,6 +503,8 @@ def run_ours(args, w):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
     value = K / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gbt)
 
     # ---- per-kernel device time for the roofline (separate profiled run of K steps) ----
     gbt.set_profiling(True)
@@ -619,6 +621,32 @@ def run_ours(args, w):
         dist.destroy_process_group()
 
 
+DUMP_MAX_PREDICTIONS = 15_000_000   # 60 MB of float32: every row of the 10M-row workloads; the tree adds < 0.1 MB
+
+
+def dump_outputs(out_dir, gbt):
+    """Writes what the last timed iteration gave its caller, as float64 / float32 .npy files in `out_dir`: the tree
+    (tree_<field>.npy, one file per field of NODE_DTYPE but threshold_value, which include/ygg_b200.h defines as NaN
+    on every node of a dataset without bucket values, as here: threshold_bin holds the split), its training loss and
+    secondary metric (train_loss.npy) and
+    the training predictions after it (predictions.npy; rank 0's rows when the rows are sharded).  Of more than
+    DUMP_MAX_PREDICTIONS predictions, those of DUMP_MAX_PREDICTIONS rows drawn with a fixed seed are kept, in row
+    order: the same rows in every run with the same number of rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    it = gbt.num_trees() - 1
+    tree = gbt.get_tree(it)
+    for k in tree.dtype.names:
+        if k == "threshold_value":
+            continue
+        np.save(os.path.join(out_dir, f"tree_{k}.npy"), tree[k].astype(np.float64))
+    np.save(os.path.join(out_dir, "train_loss.npy"), np.array(gbt.train_loss(it), np.float64))
+    pred = gbt.get_predictions()
+    if len(pred) > DUMP_MAX_PREDICTIONS:
+        pred = pred[np.sort(np.random.default_rng(0).choice(len(pred), DUMP_MAX_PREDICTIONS, replace=False))]
+    np.save(os.path.join(out_dir, "predictions.npy"), pred.astype(np.float32))
+    log(f"bench.py: outputs of iteration {it} written to {out_dir}")
+
+
 def parity_trees(args, w):
     """Trees compared with the oracle in the same run: 20 at C2 (SURVEY.md §8d), 2 at the 10M-row workloads (a CPU
     iteration takes seconds there)."""
@@ -677,7 +705,14 @@ def main():
                          "torch.distributed from Python callbacks (A/B)")
     ap.add_argument("--shard", default="rows", choices=["rows", "features"],
                     help="multi-GPU decomposition: rows (histogram all-reduce) or features (best-split all-gather)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the tree, training loss and predictions of the last timed iteration to DIR as .npy "
+                         "(at most 64 MB), to compare two builds on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     w = dict(WORKLOADS[args.workload])
     if args.rows:
         w["rows"] = args.rows

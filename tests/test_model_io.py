@@ -9,7 +9,6 @@ import ydf_b200
 from ydf_b200 import dataspec, model_io
 from ydf_b200.model import GradientBoostedTreesModel
 
-REF_GOLDEN = "/root/reference/yggdrasil_decision_forests/test_data/golden/gbt_abalone"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -54,20 +53,25 @@ def test_write_and_read_back(tmp_path, hessian):
     assert r["created_num_rows"] == 10
 
 
-def test_reader_parses_reference_format_fixture():
-    """tests/golden/ydf_gbt_abalone_head.npz holds the first tree of the reference's golden model
-    test_data/golden/gbt_abalone as decoded by this reader when /root/reference was mounted
-    (tests/golden/make_ydf_format_fixture.py).  When the reference is mounted, re-decode and compare."""
+def test_reader_parses_reference_format_fixture(tmp_path):
+    """tests/golden/ydf_gbt_abalone_head.npz holds the files of the reference's golden model test_data/golden/gbt_abalone
+    (file_<name>) and the head of that model as this reader decoded it (tests/golden/make_ydf_format_fixture.py).
+    The files are decoded again and compared with the stored head."""
     fx = np.load(os.path.join(HERE, "golden", "ydf_gbt_abalone_head.npz"), allow_pickle=False)
     assert fx["node_format"] == "BLOB_SEQUENCE" and int(fx["num_trees"]) == 42 and int(fx["loss"]) == 2
     assert int(fx["root_n"]) == 1908 and int(fx["root_n_pos"]) == 1189
     # pre-order with the negative child first: node 1 holds the n - n_pos rows of the root
     assert int(fx["node1_n"]) == 1908 - 1189
-    if os.path.isdir(REF_GOLDEN):
-        r = model_io.read_ydf_model(REF_GOLDEN)
-        assert r["num_trees"] == 42 and r["nodes"][0]["n"] == 1908 and r["nodes"][0]["n_pos"] == 1189
-        assert abs(r["nodes"][0]["higher_threshold"] - float(fx["root_threshold"])) == 0
-        assert len(r["nodes"]) == int(fx["num_nodes"])
+    d = tmp_path / "gbt_abalone"
+    d.mkdir()
+    for k in fx.files:
+        if k.startswith("file_"):
+            (d / k[5:]).write_bytes(fx[k].tobytes())
+    r = model_io.read_ydf_model(str(d))
+    assert r["num_trees"] == 42 and r["nodes"][0]["n"] == 1908 and r["nodes"][0]["n_pos"] == 1189
+    assert abs(r["nodes"][0]["higher_threshold"] - float(fx["root_threshold"])) == 0
+    assert len(r["nodes"]) == int(fx["num_nodes"])
+    assert r["initial_predictions"][0] == fx["initial_prediction"] and r["nodes"][0]["split_score"] == fx["root_score"]
 
 
 def test_reference_golden_model_and_predictions(tmp_path):
