@@ -23,13 +23,13 @@ def _declared_symbols():
     return names
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_of_abi_4():
     L = ydf_b200.lib()
     declared = _declared_symbols()
     assert len(declared) >= 25
     for name in sorted(declared):
         assert hasattr(L, name), name
-    assert L.ygg_abi_version() == 3
+    assert L.ygg_abi_version() == 4
 
 
 def test_comm_bootstrap_without_device():
@@ -69,6 +69,27 @@ def test_argument_validation_and_loud_failure_without_device():
             ydf_b200.Dataset(np.zeros((2, 10), np.uint8), [2, 2], [0, 0])
         assert e.value.code == 2  # NO_DEVICE: there is no CPU fallback
         assert "no CPU fallback" in str(e.value)
+
+
+def test_histogram_capture_validates_arguments():
+    L = ydf_b200.lib()
+    assert L.ygg_gbt_debug_capture_histograms(None, C.c_int32(1)) == 1
+    info = _capi.HistLevelInfo()
+    assert L.ygg_gbt_debug_level_histograms(None, C.c_int32(0), C.byref(info), None, None, None, None, C.c_int32(0)) == 1
+    assert C.sizeof(_capi.HistLevelInfo) == 80   # sizeof(ygg_hist_level_info), include/ygg_b200.h
+
+
+def test_histogram_reference_quantiser():
+    """The restatement the GPU histogram tests compare with: P strictly above max|g|, clamped 24-bit codes."""
+    from tests.util import Q_BIAS, Q_MAX, g_pow2_exp, quantize_g, quantize_h2
+    assert g_pow2_exp(np.float32([0.5, -0.25])) == 0 and g_pow2_exp(np.float32([-0.5])) == 0
+    assert g_pow2_exp(np.zeros(3, np.float32)) == 0 and g_pow2_exp(np.float32([2.0 ** -140])) == -139
+    assert g_pow2_exp(np.float32([0.75])) == 0 and g_pow2_exp(np.float32([1.0])) == 1
+    below = np.nextafter(np.float32(1), np.float32(0))
+    assert quantize_g(np.float32([0.5, -0.5, 0.0, below, -below]), 0).tolist() == \
+        [Q_BIAS + (1 << 22), Q_BIAS - (1 << 22), Q_BIAS, Q_MAX, 0]
+    assert quantize_g(np.float32([2.0 ** -120]), -119).tolist() == [Q_BIAS + (1 << 22)]
+    assert quantize_h2(np.float32([0.25, 0.125, 0.0]), 0.25).tolist() == [1 << 24, 1 << 23, 0]
 
 
 def test_learner_rejects_options_outside_the_path():

@@ -24,12 +24,12 @@ def _build(tmp_path):
     return exe
 
 
-def test_example_fails_loudly_without_a_device(tmp_path):
+def test_example_reports_abi_4_and_fails_loudly_without_a_device(tmp_path):
     if ydf_b200.device_count() > 0:
         pytest.skip("a CUDA device is present")
     r = subprocess.run([_build(tmp_path), "1000", "4", "5"], capture_output=True, text=True)
     assert r.returncode == 2                                        # YGG_ERR_NO_DEVICE
-    assert "no CPU fallback" in r.stderr and "ABI 3" in r.stdout
+    assert "no CPU fallback" in r.stderr and "ABI 4" in r.stdout
 
 
 @pytest.mark.gpu

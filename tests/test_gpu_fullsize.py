@@ -1,11 +1,12 @@
 """Size-independent properties at BASELINE.json's full size (C3: 10M rows x 200 features, 256 bins,
 depth 8), where the CPU oracle would take minutes per tree: conservation of row counts and of the
 fixed-point sums across every split, exactness of sibling subtraction, run-to-run determinism,
-monotone training loss, and a spot check of the root histogram against numpy."""
+monotone training loss, and an exact check of the root histogram against numpy."""
 import numpy as np
 import pytest
 
 import ydf_b200
+from tests.util import quantize_g
 
 pytestmark = pytest.mark.gpu
 
@@ -51,7 +52,7 @@ def _check_tree(t, n_rows):
     assert len(t) <= 2 ** W["max_depth"] - 1
 
 
-def test_full_size_properties(data):
+def test_full_size_properties_and_exact_root_histogram(data):
     bins, nb, na, y = data
     n = bins.shape[1]
     ds, gbt, trees, losses = _train(data, 3)
@@ -66,16 +67,18 @@ def test_full_size_properties(data):
     assert [t.tobytes() for t in trees] == [t.tobytes() for t in trees2]
     assert losses == losses2
     assert pred.tobytes() == gbt2.get_predictions().tobytes()
-    # root histogram of two features against numpy (counts exact, sums within the 24-bit quantisation)
+    # root histogram of two features against numpy, bin for bin
     rng = np.random.default_rng(0)
-    g = rng.normal(size=n).astype(np.float32)
-    node_of_row = np.zeros(n, np.int32)
+    g = (rng.uniform(-1, 1, size=n) * 0.999).astype(np.float32)   # binomial: P = 1
+    gbt2.debug_capture_histograms(True)
+    gbt2.train_tree_on_gradients(g, np.full(n, 0.25, np.float32))
+    root = gbt2.debug_level_histograms(0)
+    assert root["layout"] == "root_sum" and root["g_pow2"] == 1.0 and root["num_slots"] == 1
+    q = quantize_g(g, 0)
     for f in (0, 199):
-        s, c = gbt2.debug_histogram(g, node_of_row, 0, f)
-        want_c = np.bincount(bins[f], minlength=nb[f])
-        want_s = np.bincount(bins[f], weights=g.astype(np.float64), minlength=nb[f])
-        np.testing.assert_array_equal(c, want_c)
-        P = 2.0 ** np.ceil(np.log2(np.abs(g).max()))
-        assert np.all(np.abs(s - want_s) <= want_c * P * 2.0 ** -24 + 1e-9)
-        assert c.sum() == n
+        want_c = np.bincount(bins[f], minlength=256)
+        want_s = np.bincount(bins[f], weights=q, minlength=256).astype(np.int64)
+        np.testing.assert_array_equal(root["cnt"][0, f], want_c)
+        np.testing.assert_array_equal(root["sum"][0, f].astype(np.int64), want_s)
+        assert root["cnt"][0, f].sum() == n
     gbt2.close(); ds2.close()

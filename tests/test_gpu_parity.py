@@ -8,7 +8,7 @@ import pytest
 
 import ydf_b200
 from oracle import oracle as O
-from tests.util import compare_trees, first_divergence, synth
+from tests.util import check_captured_levels, compare_trees, first_divergence, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -85,21 +85,18 @@ def test_partition_rows_matches_oracle(n):
 
 
 @pytest.mark.parametrize("n", [5000, 70000])
-def test_histogram_matches_numpy(n):
+def test_level_histograms_match_numpy(n):
+    """Every level histogram of a grown tree equals the numpy restatement bin for bin (tests/test_gpu_hist_exact.py
+    holds each layout to it)."""
     bins, nb, na, y = synth(n, 4, seed=3)
-    ds, gbt, cfg = _mk(bins, nb, na)
+    ds, gbt, cfg = _mk(bins, nb, na, loss=1, max_depth=4)
     rng = np.random.default_rng(0)
     g = rng.normal(size=n).astype(np.float32)
-    node_of_row = rng.integers(0, 3, size=n).astype(np.int32)
-    for f in (0, 3):
-        s, c = gbt.debug_histogram(g, node_of_row, 1, f)
-        m = node_of_row == 1
-        want_c = np.bincount(bins[f][m], minlength=nb[f])
-        want_s = np.bincount(bins[f][m], weights=g[m].astype(np.float64), minlength=nb[f])
-        np.testing.assert_array_equal(c, want_c)
-        # 24-bit fixed point: |err| <= count * P * 2^-24
-        P = 2.0 ** np.ceil(np.log2(np.abs(g).max()))
-        assert np.all(np.abs(s - want_s) <= want_c * P * 2.0 ** -24 + 1e-12)
+    gbt.debug_capture_histograms(True)
+    tree = gbt.train_tree_on_gradients(g)
+    assert len(tree) > 7
+    caps = check_captured_levels(gbt, tree, bins, ["root_sum", "packed", "packed"])
+    assert caps[0]["cnt"][0].sum(axis=1).tolist() == [n] * 4
 
 
 CASES = [

@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests: synthetic data (SURVEY.md §8d generator), tree comparison."""
+import math
+
 import numpy as np
 
 
@@ -181,3 +183,108 @@ def predict_raw(trees, initial_prediction, bins):
             node[act] = np.where(go, t["pos_child"][nd], t["neg_child"][nd])
         raw += t["leaf_value"][node]
     return raw
+
+
+# ---- exact restatement of the level histograms (ygg_gbt_debug_level_histograms) --------------------------------
+
+Q_BIAS = 1 << 23
+Q_MAX = (1 << 24) - 1
+
+
+def g_pow2_exp(g):
+    """e of P = 2^e, the smallest power of two strictly above max|g| (P = 1 when every g is 0)."""
+    m = float(np.max(np.abs(g.astype(np.float64)))) if len(g) else 0.0
+    return 0 if m == 0.0 else math.frexp(m)[1]   # m = f * 2^e, 0.5 <= f < 1: 2^(e-1) <= m < 2^e
+
+
+def quantize_g(g, e):
+    """q = clip(rint(g * 2^(23-e)) + 2^23, 0, 2^24 - 1), exact in float64 (a power-of-two scale of a float32)."""
+    t = np.rint(g.astype(np.float32).astype(np.float64) * 2.0 ** (23 - e)) + Q_BIAS
+    return np.clip(t, 0, Q_MAX).astype(np.int64)
+
+
+def quantize_h2(v, h2_pow2):
+    """The second plane (hessians or weights): [0, 2^24] inclusive."""
+    return np.minimum(np.rint(v.astype(np.float32).astype(np.float64) * (2.0 ** 24 / float(h2_pow2))), 1 << 24).astype(np.int64)
+
+
+def node_per_level(tree, bins, levels):
+    """[levels, n]: the node (index in `tree`) each row sits in at every level, -1 once it has reached a leaf."""
+    n = bins.shape[1]
+    rows = np.arange(n)
+    node = np.zeros(n, np.int64)
+    alive = np.ones(n, bool)
+    out = np.full((levels, n), -1, np.int64)
+    for l in range(levels):
+        out[l, alive] = node[alive]
+        f = tree["feature"][node]
+        alive &= f >= 0
+        act = np.nonzero(alive)[0]
+        nd = node[act]
+        v = bins[f[act], rows[act]].astype(np.int64)
+        in_set = ((tree["cat_mask"][nd, v >> 5] >> (v & 31).astype(np.uint32)) & 1) != 0
+        go = np.where(tree["condition_type"][nd] == 1, in_set, v >= tree["threshold_bin"][nd])
+        node[act] = np.where(go, tree["pos_child"][nd], tree["neg_child"][nd])
+    return out
+
+
+def expected_planes(cap, tree, bins, node_at_level, q, hq=None):
+    """int64 [slot, feature, 256] sums of q, hq and counts over the rows of every slot's node (sampled rows only)."""
+    S, F = cap["num_slots"], cap["num_features"]
+    slot_of_node = np.full(len(tree), -1, np.int64)
+    slot_of_node[cap["slot_node"]] = np.arange(S)
+    rs = np.where(node_at_level >= 0, slot_of_node[np.maximum(node_at_level, 0)], -1)
+    rs[~cap["selected"]] = -1
+    m = rs >= 0
+    out = {k: np.zeros((S, F, 256), np.int64) for k in ("sum", "hsum", "cnt")}
+    for fl in range(F):
+        key = rs[m] * 256 + bins[cap["feature_begin"] + fl][m].astype(np.int64)
+        out["cnt"][:, fl] = np.bincount(key, minlength=S * 256).reshape(S, 256)
+        # float64 bincount weights are exact here: every sum stays below 2^53
+        out["sum"][:, fl] = np.bincount(key, weights=q[m], minlength=S * 256).reshape(S, 256).astype(np.int64)
+        if hq is not None:
+            out["hsum"][:, fl] = np.bincount(key, weights=hq[m], minlength=S * 256).reshape(S, 256).astype(np.int64)
+    return out
+
+
+def _first_diff(name, got, want):
+    bad = np.argwhere(got.astype(np.int64) != want)
+    s, f, b = bad[0]
+    return (f"{name}: {len(bad)} bins differ, first at slot {s} feature {f} bin {b}: "
+            f"{int(got[s, f, b])} != {int(want[s, f, b])}")
+
+
+def check_captured_levels(gbt, tree, bins, layouts, g_pow2=None, h2_pow2=None):
+    """Compares every level of the last tree `gbt` grew with the histogram capture on (Gbt.debug_capture_histograms)
+    with the numpy restatement, for equality.  layouts[l] = the layout level l must have run with (None: not asserted);
+    there must be exactly len(layouts) levels.  g_pow2 / h2_pow2: the scales the planes must have used (default for
+    g_pow2: the smallest power of two strictly above max|g|).  Returns the captures."""
+    import ydf_b200
+    caps = [gbt.debug_level_histograms(l) for l in range(len(layouts))]
+    try:
+        gbt.debug_level_histograms(len(layouts))
+        raise AssertionError(f"more than {len(layouts)} histogram levels were captured")
+    except ydf_b200.YggError:
+        pass
+    c0 = caps[0]
+    # P: the smallest power of two above max|g| over all rows of the iteration (sampled or not); the binomial loss
+    # without weights has |g| <= 1 and uses P = 1: the caller passes g_pow2 = 1
+    want_p = 2.0 ** g_pow2_exp(c0["g"]) if g_pow2 is None else g_pow2
+    assert c0["g_pow2"] == want_p, (c0["g_pow2"], want_p)
+    if h2_pow2 is not None:
+        assert c0["h2_pow2"] == h2_pow2
+    q = quantize_g(c0["g"], int(round(math.log2(c0["g_pow2"]))))
+    hq = quantize_h2(c0["h2"], c0["h2_pow2"]) if c0["has_hsum"] else None
+    at = node_per_level(tree, bins, len(layouts))
+    for l, cap in enumerate(caps):
+        if layouts[l] is not None:
+            assert cap["layout"] == layouts[l], (l, cap["layout"], layouts[l], cap)
+        want = expected_planes(cap, tree, bins, at[l], q, hq)
+        assert np.array_equal(cap["cnt"], want["cnt"]), f"level {l}: " + _first_diff("cnt", cap["cnt"], want["cnt"])
+        assert np.array_equal(cap["sum"], want["sum"]), f"level {l}: " + _first_diff("sum", cap["sum"], want["sum"])
+        if hq is not None:
+            assert np.array_equal(cap["hsum"], want["hsum"]), f"level {l}: " + _first_diff("hsum", cap["hsum"], want["hsum"])
+        # cross-check with the partition: every feature of a slot counts its node's rows
+        per_feature = cap["cnt"].astype(np.int64).sum(axis=2)
+        assert np.array_equal(per_feature, np.repeat(tree["num_examples"][cap["slot_node"]][:, None], cap["num_features"], 1))
+    return caps

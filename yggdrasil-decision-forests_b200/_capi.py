@@ -43,6 +43,18 @@ assert NODE_DTYPE.itemsize == 112  # sizeof(ygg_node), include/ygg_b200.h
 FEATURE_DISCRETIZED_NUMERICAL = 0
 FEATURE_CATEGORICAL = 1
 
+# enum ygg_hist_layout
+HIST_LAYOUTS = ("root_sum", "packed", "shared", "shared_hess", "packed_multi", "shared_multi", "shared_hess_multi", "hist2")
+
+
+class HistLevelInfo(C.Structure):
+    _fields_ = [
+        ("layout", C.c_int32), ("features_per_item", C.c_int32), ("smem_slots", C.c_int32), ("passes", C.c_int32),
+        ("chunk_blocks", C.c_int32), ("hist2_lanes", C.c_int32), ("num_slots", C.c_int32), ("feature_begin", C.c_int32),
+        ("num_features", C.c_int32), ("has_hsum", C.c_int32), ("g_pow2", C.c_float), ("h2_pow2", C.c_float),
+        ("n_rows", C.c_int64), ("g", C.POINTER(C.c_float)), ("h2", C.POINTER(C.c_float)), ("selected", C.POINTER(C.c_uint8)),
+    ]
+
 ALLGATHER_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p)
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p)
 REDUCESCATTER_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p)
@@ -55,7 +67,7 @@ EXPORTS = [
     "ygg_merge_shard_best", "ygg_gbt_initial_prediction",
     "ygg_gbt_train", "ygg_gbt_train_timed", "ygg_gbt_step", "ygg_gbt_sync", "ygg_gbt_num_trees", "ygg_gbt_get_tree",
     "ygg_gbt_train_loss", "ygg_gbt_get_predictions", "ygg_gbt_set_predictions", "ygg_gbt_predict",
-    "ygg_tree_train_on_gradients", "ygg_debug_histogram", "ygg_partition_rows",
+    "ygg_tree_train_on_gradients", "ygg_gbt_debug_capture_histograms", "ygg_gbt_debug_level_histograms", "ygg_partition_rows",
     "ygg_gbt_set_profiling", "ygg_gbt_get_profile", "ygg_gbt_save_ydf",
     "ygg_discretize_boundaries", "ygg_discretize_encode", "ygg_model_write_ydf",
     "ygg_validation_split_mask", "ygg_dataset_split_rows", "ygg_gbt_set_validation_i32",
@@ -556,16 +568,32 @@ class Gbt:
                                                 C.byref(n)))
         return out[:n.value].copy()
 
-    def debug_histogram(self, g, node_of_row, node, feature):
-        g = np.ascontiguousarray(g, dtype=np.float32)
-        nor = np.ascontiguousarray(node_of_row, dtype=np.int32)
-        nb = int(self.dataset.num_bins[feature])
-        s = np.zeros(nb, dtype=np.float64)
-        c = np.zeros(nb, dtype=np.int64)
-        check(lib().ygg_debug_histogram(self.handle, ptr(g, C.c_float), ptr(nor, C.c_int32),
-                                        C.c_int32(node), C.c_int32(feature), ptr(s, C.c_double),
-                                        ptr(c, C.c_int64)))
-        return s, c
+    def debug_capture_histograms(self, enabled=True):
+        """While enabled, every tree grown records the slot histograms of each of its levels (debug_level_histograms)."""
+        check(lib().ygg_gbt_debug_capture_histograms(self.handle, C.c_int32(int(enabled))))
+
+    def debug_level_histograms(self, level):
+        """The capture of `level` of the last tree grown with the capture on -> dict: the launch configuration
+        (ygg_hist_level_info, "layout" as a name of HIST_LAYOUTS), the quantiser's inputs "g", "h2", "selected" [n_rows],
+        and the planes "sum", "hsum" (None without a second plane), "cnt" as [slot, feature, 256] arrays (uint64 / uint32)
+        with "slot_node" [slot] = the slot's node in the returned tree array."""
+        info = HistLevelInfo()
+        check(lib().ygg_gbt_debug_level_histograms(self.handle, C.c_int32(level), C.byref(info), None, None, None, None,
+                                                   C.c_int32(0)))
+        n, S, F = info.n_rows, info.num_slots, info.num_features
+        g, h2, sel = np.empty(n, np.float32), np.empty(n, np.float32), np.empty(n, np.uint8)
+        info.g, info.h2, info.selected = ptr(g, C.c_float), ptr(h2, C.c_float), ptr(sel, C.c_uint8)
+        s = np.zeros((S, F, 256), np.uint64)
+        hs = np.zeros((S, F, 256), np.uint64) if info.has_hsum else None
+        c = np.zeros((S, F, 256), np.uint32)
+        sn = np.zeros(S, np.int32)
+        check(lib().ygg_gbt_debug_level_histograms(self.handle, C.c_int32(level), C.byref(info), ptr(s, C.c_uint64),
+                                                   ptr(hs, C.c_uint64), ptr(c, C.c_uint32), ptr(sn, C.c_int32),
+                                                   C.c_int32(S)))
+        out = {k: getattr(info, k) for k, _ in HistLevelInfo._fields_ if k not in ("g", "h2", "selected")}
+        out["layout"] = HIST_LAYOUTS[info.layout]
+        out.update(g=g, h2=h2, selected=sel.astype(bool), sum=s, hsum=hs, cnt=c, slot_node=sn)
+        return out
 
     def set_profiling(self, enabled=True):
         check(lib().ygg_gbt_set_profiling(self.handle, C.c_int32(int(enabled))))

@@ -234,6 +234,18 @@ struct ygg_gbt {
   int hist2_FL[32]{}, hist2_T[32]{};   // > 0: the level runs k_hist2 with FL feature lanes and T sub-tiles per tile
   size_t hist_smem[32]{};
   int part_smem_children = 0;
+  // histogram capture (ygg_gbt_debug_capture_histograms): every level's slot planes of the last tree grown
+  bool capture_hist = false;
+  unsigned long long* d_capture = nullptr;   // level l's level buffer at capture_off[l]
+  size_t capture_u64 = 0;
+  std::vector<size_t> capture_off;
+  std::vector<ygg_hist_level_info> capture_info;   // launch configuration of every captured level
+  float* d_capture_g = nullptr;      // [n_pad] the quantiser's inputs: gradients,
+  float* d_capture_h2 = nullptr;     // [n_pad] the second plane's values (hessians or weights),
+  uint8_t* d_capture_sel = nullptr;  // [n_pad] the sampled rows
+  bool capture_has_h2 = false, capture_has_sel = false;
+  DeviceState* d_capture_st = nullptr;
+  const NodeRec* capture_nodes = nullptr;   // node table of the captured tree (null: nothing captured)
   // profiling
   bool profiling = false;
   std::map<std::string, ProfileSlot> profile;
@@ -395,7 +407,6 @@ int for_hist_kernel(bool hess, int mode, F f, bool multi = false) {
   }
   if (hess) return f(k_hist<true, kHistShared>);
   if (mode == kHistRootSum) return f(k_hist<false, kHistRootSum>);
-  if (mode == kHistPrivate) return f(k_hist<false, kHistPrivate>);
   if (mode == kHistPacked) return f(k_hist<false, kHistPacked>);
   return f(k_hist<false, kHistShared>);
 }
@@ -465,12 +476,10 @@ int configure_launches(ygg_gbt* h) {
     h->hist_mode[l] = mode;
     h->hist_smem[l] = hist_smem_bytes(G, S, hh, mode);
   }
-  for (int mode = 0; mode < 4; mode++) {
+  for (int mode = 0; mode < kHistModes; mode++) {
     size_t max_smem = 0;
     for (int l = 0; l < h->num_levels; l++)
       if (h->hist_mode[l] == mode) max_smem = std::max(max_smem, h->hist_smem[l]);
-    // the debug seam runs the private layout on level-0 geometry
-    if (mode == kHistPrivate && !hh) max_smem = std::max(max_smem, hist_smem_bytes(1, 1, false, kHistPrivate));
     if (mode == kHistPacked && !hh) max_smem = std::max<size_t>(max_smem, 1);  // a level may fall back to / from it
     if (mode == kHistShared && !hh) max_smem = std::max<size_t>(max_smem, 1);
     if (max_smem == 0) continue;
@@ -496,8 +505,14 @@ int configure_launches(ygg_gbt* h) {
     const char* v = std::getenv("YGG_HIST2_ITEMS_PER_CTA");
     return v ? std::atof(v) : 0.9;
   }();
+  // YGG_HIST_CHUNK_BLOCKS=c (tests: reach the chunk sizes where the bin counters come closest to their limits) forces
+  // c row blocks per work item, clamped to [step, kHistMaxChunkBlocks] and rounded down to the step.  Read at every
+  // configure, like YGG_HIST2.
+  const char* env_chunk = std::getenv("YGG_HIST_CHUNK_BLOCKS");
+  const int forced_chunk = env_chunk != nullptr ? std::atoi(env_chunk) : 0;
   auto choose_chunk = [&](int n_fgroups, int grid, int step, double need) {
     const int max_c = std::max(step, kHistMaxChunkBlocks / step * step);
+    if (forced_chunk > 0) return std::max(step, std::min(forced_chunk, max_c) / step * step);
     const int min_chunks = std::max(1, (n_blocks + max_c - 1) / max_c);
     int best = max_c;
     double best_score = -1;
@@ -632,8 +647,6 @@ int allocate_level_buffers(ygg_gbt* h) {
     const int stats_nodes = l == 0 ? 1 : (2 << (l - 1));
     max_u64 = std::max(max_u64, level_buf(h, slots, stats_nodes).total_u64);
   }
-  // debug seam: one slot over the hist features
-  max_u64 = std::max(max_u64, level_buf(h, 1, 1).total_u64);
   (void)f_hist;
   h->level_buf_bytes = max_u64 * sizeof(unsigned long long);
   YGG_RETURN_IF_ERROR(dev_alloc_plain(&h->d_level_buf, max_u64));
@@ -717,6 +730,62 @@ int launch_weight_sums(ygg_gbt* h, NodeRec* nodes) {
   return check_launch("k_weight_sums");
 }
 
+// Histogram capture: sizes the buffers for this handle's level geometry and records the launch configuration of every
+// level and the quantiser's float inputs `q` of the tree about to be grown.
+int begin_capture(ygg_gbt* h, const QuantParams& q) {
+  h->capture_nodes = nullptr;
+  h->capture_off.assign(h->num_levels, 0);
+  size_t total = 0;
+  for (int l = 0; l < h->num_levels; l++) {
+    h->capture_off[l] = total;
+    total += level_buf(h, level_slot_bound(h, l), l == 0 ? 1 : (2 << (l - 1))).total_u64;
+  }
+  if (h->d_capture == nullptr || h->capture_u64 < total) {
+    YGG_CUDA(cudaStreamSynchronize(h->stream));
+    dev_free(h->d_capture);
+    h->d_capture = nullptr;
+    YGG_RETURN_IF_ERROR(dev_alloc(&h->d_capture, total));
+    h->capture_u64 = total;
+  }
+  const int64_t n_pad = h->ds->n_pad;
+  if (h->d_capture_st == nullptr) {
+    YGG_RETURN_IF_ERROR(dev_alloc(&h->d_capture_st, 1));
+    YGG_RETURN_IF_ERROR(dev_alloc(&h->d_capture_g, n_pad));
+    YGG_RETURN_IF_ERROR(dev_alloc(&h->d_capture_h2, n_pad));
+    YGG_RETURN_IF_ERROR(dev_alloc(&h->d_capture_sel, n_pad));
+  }
+  const int64_t n = h->ds->n;
+  const float* h2 = q.hist_h != nullptr ? q.hist_h : q.h;
+  h->capture_has_h2 = h2 != nullptr;
+  h->capture_has_sel = q.selected != nullptr;
+  YGG_CUDA(cudaMemcpyAsync(h->d_capture_g, q.g, n * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
+  if (h2 != nullptr) YGG_CUDA(cudaMemcpyAsync(h->d_capture_h2, h2, n * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
+  if (q.selected != nullptr)
+    YGG_CUDA(cudaMemcpyAsync(h->d_capture_sel, q.selected, n * sizeof(uint8_t), cudaMemcpyDeviceToDevice, h->stream));
+  h->capture_info.assign(h->num_levels, ygg_hist_level_info{});
+  const bool hess = hist_hess(h);
+  for (int l = 0; l < h->num_levels; l++) {
+    ygg_hist_level_info& in = h->capture_info[l];
+    const bool multi = h->hist_passes[l] > 1;
+    if (h->hist2_FL[l] > 0) in.layout = YGG_HIST_LAYOUT_HIST2;
+    else if (hess) in.layout = multi ? YGG_HIST_LAYOUT_SHARED_HESS_MULTI : YGG_HIST_LAYOUT_SHARED_HESS;
+    else if (h->hist_mode[l] == kHistRootSum) in.layout = YGG_HIST_LAYOUT_ROOT_SUM;
+    else if (h->hist_mode[l] == kHistPacked) in.layout = multi ? YGG_HIST_LAYOUT_PACKED_MULTI : YGG_HIST_LAYOUT_PACKED;
+    else in.layout = multi ? YGG_HIST_LAYOUT_SHARED_MULTI : YGG_HIST_LAYOUT_SHARED;
+    in.features_per_item = h->hist2_FL[l] > 0 ? 0 : h->hist_G[l];
+    in.smem_slots = h->hist_S[l];
+    in.passes = h->hist_passes[l];
+    in.chunk_blocks = h->hist_chunk[l];
+    in.hist2_lanes = h->hist2_FL[l];
+    in.feature_begin = h->hist_f_begin;
+    in.num_features = h->hist_f_end - h->hist_f_begin;
+    in.has_hsum = hess ? 1 : 0;
+    in.h2_pow2 = q.hist_h != nullptr ? q.hist_h_pow2 : q.h_pow2;
+    in.n_rows = n;
+  }
+  return YGG_OK;
+}
+
 // Grows one tree on the gradients currently in d_g / d_h (gmax_bits must already be in d_st and the
 // iteration scalars reset).  Everything is enqueued on h->stream; no host sync.
 //
@@ -760,6 +829,7 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
       YGG_RETURN_IF_ERROR(check_launch("k_compact_root"));
     }
     if (h->num_levels > 0) YGG_RETURN_IF_ERROR(replicate_stats(h, lb0, 1));
+    if (h->capture_hist) YGG_RETURN_IF_ERROR(begin_capture(h, q));
   }
   StatsParams sp{};
   sp.levels = h->d_levels; sp.nodes = nodes; sp.st = h->d_st;
@@ -836,6 +906,9 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
       }
       }
     }
+    if (h->capture_hist)   // this rank's own planes, before any collective
+      YGG_CUDA(cudaMemcpyAsync(h->d_capture + h->capture_off[l], h->d_level_buf, lb.total_u64 * sizeof(unsigned long long),
+                               cudaMemcpyDeviceToDevice, h->stream));
     // after the collective this rank's statistics of the level sit in `level_stats`
     const unsigned long long* level_stats = lb.stats;
     if (rows_sharded && h->scatter) {
@@ -954,6 +1027,10 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
     }
   }
   if (weighted(h)) YGG_RETURN_IF_ERROR(launch_weight_sums(h, nodes));
+  if (h->capture_hist) {
+    YGG_CUDA(cudaMemcpyAsync(h->d_capture_st, h->d_st, sizeof(DeviceState), cudaMemcpyDeviceToDevice, h->stream));
+    h->capture_nodes = nodes;
+  }
   if (h->cfg.candidate_shuffle != 0 && h->world == 1) {
     // which of the tied candidates recorded by k_select_local cut their node's rows exactly like the chosen split
     ProfScope ps(h, "select");
@@ -989,27 +1066,6 @@ __global__ void k_absmax(const float* g, int64_t n, DeviceState* st) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
   if ((threadIdx.x & 31) == 0) atomicMax(&st->gmax_bits, __float_as_uint(m));
-}
-
-// Debug seam: dense "active list" selecting the rows of one node (inactive rows get count 0 by
-// being routed to slot 0 with... no: they are simply left out block by block on the host side of the
-// list, so this kernel builds the list with a per-block serial compaction — test sizes only).
-__global__ void k_debug_actlists(const float* g, const int32_t* node_of_row, int node, int64_t n, int n_blocks,
-                                 const DeviceState* st, uint2* act, int32_t* act_count) {
-  const float P = pow2_cover(st->gmax_bits);
-  const float qscale = static_cast<float>(1u << (kQBits - 1)) / P;
-  for (int blk = blockIdx.x * blockDim.x + threadIdx.x; blk < n_blocks; blk += gridDim.x * blockDim.x) {
-    int cnt = 0;
-    const int64_t base = static_cast<int64_t>(blk) * kBlockRows;
-    for (int j = 0; j < kBlockRows; j++) {
-      const int64_t r = base + j;
-      if (r < n && node_of_row[r] == node) {
-        act[base + cnt] = make_uint2(quant_biased(g[r], qscale, kQBias, kQMax), static_cast<uint32_t>(j));
-        cnt++;
-      }
-    }
-    act_count[blk] = cnt;
-  }
 }
 
 // Runs the pred/grad kernel.  apply: add the pending tree to the predictions and account its loss.
@@ -1558,6 +1614,14 @@ int best_first_prune(ygg_gbt* h, NodeRec* d_tree) {
   return YGG_OK;
 }
 
+// Position of every node id in preorder()'s output (-1: not in the tree).
+void preorder_positions(const std::vector<NodeRec>& nodes, int idx, int* next, std::vector<int>* pos) {
+  (*pos)[idx] = (*next)++;
+  if (nodes[idx].feature < 0) return;
+  preorder_positions(nodes, nodes[idx].neg_child, next, pos);
+  preorder_positions(nodes, nodes[idx].pos_child, next, pos);
+}
+
 void preorder(const std::vector<NodeRec>& nodes, int idx, std::vector<ygg_node>* out) {
   const NodeRec& n = nodes[idx];
   const int my = static_cast<int>(out->size());
@@ -1914,6 +1978,7 @@ int ygg_gbt_destroy(ygg_gbt* h) {
   dev_free(h->d_weight); dev_free(h->d_g2w); dev_free(h->d_wsums); dev_free(h->d_vweight);
   for (int i = 0; i < 2; i++) { dev_free(h->d_goss_keys[i]); dev_free(h->d_goss_rows[i]); }
   dev_free(h->d_goss_u);
+  dev_free(h->d_capture); dev_free(h->d_capture_g); dev_free(h->d_capture_h2); dev_free(h->d_capture_sel); dev_free(h->d_capture_st);
   cudaFree(h->d_goss_temp);
   cudaFree(h->d_level_buf);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -2629,62 +2694,74 @@ int ygg_tree_train_on_gradients(ygg_gbt* h, const float* gradients, const float*
   return YGG_OK;
 }
 
-int ygg_debug_histogram(ygg_gbt* h, const float* gradients, const int32_t* node_of_row, int32_t node,
-                        int32_t feature, double* out_sum, int64_t* out_count) {
-  if (!h || !gradients || !node_of_row || !out_sum || !out_count) return set_error(YGG_ERR_INVALID_ARGUMENT, "null argument");
-  if (feature < h->hist_f_begin || feature >= h->hist_f_end) return set_error(YGG_ERR_INVALID_ARGUMENT, "feature %d outside this shard", feature);
+int ygg_gbt_debug_capture_histograms(ygg_gbt* h, int32_t enabled) {
+  if (!h) return set_error(YGG_ERR_INVALID_ARGUMENT, "null handle");
+  h->capture_hist = enabled != 0;
+  return YGG_OK;
+}
+
+int ygg_gbt_debug_level_histograms(ygg_gbt* h, int32_t level, ygg_hist_level_info* info, uint64_t* sum, uint64_t* hsum,
+                                   uint32_t* cnt, int32_t* slot_node, int32_t capacity) {
+  if (!h || !info) return set_error(YGG_ERR_INVALID_ARGUMENT, "null argument");
+  if (h->capture_nodes == nullptr) return set_error(YGG_ERR_INVALID_ARGUMENT, "no tree was grown with the histogram capture on");
+  if (level < 0 || level >= static_cast<int>(h->capture_info.size()))
+    return set_error(YGG_ERR_INVALID_ARGUMENT, "level %d: the captured tree has %zu histogram levels", level, h->capture_info.size());
   YGG_CUDA(cudaSetDevice(h->ds->device));
-  (void)cudaGetLastError();  // stale foreign error, see ygg_gbt_step
-  YGG_RETURN_IF_ERROR(apply_pending(h));
-  const int64_t n = h->ds->n;
-  int32_t* d_nor = nullptr;
-  YGG_RETURN_IF_ERROR(dev_alloc(&d_nor, n));
-  YGG_CUDA(cudaMemcpyAsync(h->d_g, gradients, n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  YGG_CUDA(cudaMemcpyAsync(d_nor, node_of_row, n * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
-  k_begin_iteration<<<1, 1, 0, h->stream>>>(h->d_st, h->d_levels, h->d_fam[0], h->d_slot_node[0], 1);
-  h->launches_total++;
-  k_absmax<<<elementwise_grid(h), 256, 0, h->stream>>>(h->d_g, n, h->d_st);
-  h->launches_total++;
-  k_debug_actlists<<<(h->n_blocks + 63) / 64, 64, 0, h->stream>>>(h->d_g, d_nor, node, n, h->n_blocks, h->d_st,
-                                                                   h->d_act, h->d_act_count);
-  h->launches_total++;
-  YGG_RETURN_IF_ERROR(check_launch("k_debug_actlists"));
-  const int f_count = h->hist_f_end - h->hist_f_begin;
-  const LevelBuf lb = level_buf(h, 1, 1);
-  YGG_RETURN_IF_ERROR(zero_planes(h, lb));
-  HistParams hp{};
-  hp.bins = h->ds->d_bins; hp.n_pad = h->ds->n_pad; hp.act = h->d_act; hp.act_h = h->d_act_h; hp.q24 = h->d_q24;
-  hp.act_count = h->d_act_count; hp.n_blocks = h->n_blocks;
-  hp.f_begin = h->hist_f_begin; hp.f_count = f_count; hp.G = 1; hp.S = 1;
-  hp.chunk_blocks = h->hist_chunk[0];
-  hp.level = 0; hp.levels = h->d_levels;
-  hp.hist_sum = lb.sum; hp.hist_cnt = lb.cnt; hp.hist_hsum = lb.hsum;
-  hp.f_chunk = lb.f_chunk; hp.chunk_stride = static_cast<long long>(lb.chunk_u64);
-  const int dbg_mode = hist_hess(h) ? kHistShared : kHistPrivate;
-  if (hist_hess(h)) YGG_CUDA(cudaMemsetAsync(h->d_act_h, 0, h->ds->n_pad * sizeof(uint32_t), h->stream));
-  YGG_RETURN_IF_ERROR(launch_hist(h, hp, dbg_mode, h->hist_grid[0], hist_smem_bytes(1, 1, hist_hess(h), dbg_mode)));
-  std::vector<unsigned long long> sum(kMaxBins);
-  std::vector<uint32_t> cnt(kMaxBins);
-  DeviceState st;
-  size_t off_cnt;
-  const size_t off = slot_hist_offset(0, feature - h->hist_f_begin, 0, lb.f_chunk, static_cast<long long>(lb.chunk_u64), &off_cnt);
-  YGG_CUDA(cudaMemcpyAsync(sum.data(), lb.sum + off, sizeof(unsigned long long) * kMaxBins, cudaMemcpyDeviceToHost, h->stream));
-  YGG_CUDA(cudaMemcpyAsync(cnt.data(), lb.cnt + off_cnt, sizeof(uint32_t) * kMaxBins, cudaMemcpyDeviceToHost, h->stream));
-  YGG_CUDA(cudaMemcpyAsync(&st, h->d_st, sizeof(st), cudaMemcpyDeviceToHost, h->stream));
   YGG_CUDA(cudaStreamSynchronize(h->stream));
-  dev_free(d_nor);
-  const float P = [&]() {
-    const unsigned bits = st.gmax_bits;
-    if (bits == 0u) return 1.f;
-    const int e = static_cast<int>(bits >> 23) - 127;
-    return (bits & 0x7FFFFFu) == 0u ? std::ldexp(1.f, e) : std::ldexp(1.f, e + 1);
-  }();
-  const double inv = static_cast<double>(P) / static_cast<double>(1u << (kQBits - 1));
-  const int B = h->ds->num_bins[feature];
-  for (int b = 0; b < B; b++) {
-    out_count[b] = cnt[b];
-    out_sum[b] = (static_cast<double>(static_cast<long long>(sum[b])) - static_cast<double>(cnt[b]) * static_cast<double>(kQBias)) * inv;
+  float* in_g = info->g;
+  float* in_h2 = info->h2;
+  uint8_t* in_sel = info->selected;
+  *info = h->capture_info[level];
+  info->g = in_g; info->h2 = in_h2; info->selected = in_sel;
+  DeviceState st;
+  YGG_CUDA(cudaMemcpy(&st, h->d_capture_st, sizeof(st), cudaMemcpyDeviceToHost));
+  info->g_pow2 = st.g_pow2;
+  const int64_t n = h->ds->n;
+  if (in_g) YGG_CUDA(cudaMemcpy(in_g, h->d_capture_g, n * sizeof(float), cudaMemcpyDeviceToHost));
+  if (in_h2) {
+    if (h->capture_has_h2) YGG_CUDA(cudaMemcpy(in_h2, h->d_capture_h2, n * sizeof(float), cudaMemcpyDeviceToHost));
+    else std::fill(in_h2, in_h2 + n, 1.f);
   }
+  if (in_sel) {
+    if (h->capture_has_sel) YGG_CUDA(cudaMemcpy(in_sel, h->d_capture_sel, n, cudaMemcpyDeviceToHost));
+    else std::memset(in_sel, 1, n);
+  }
+  // slots of the level: its nodes (depth level + 1) whose histogram was accumulated from rows
+  std::vector<NodeRec> nodes(h->max_nodes);
+  YGG_CUDA(cudaMemcpy(nodes.data(), h->capture_nodes, sizeof(NodeRec) * h->max_nodes, cudaMemcpyDeviceToHost));
+  std::vector<int> pos(h->max_nodes, -1);
+  int next = 0;
+  preorder_positions(nodes, 0, &next, &pos);
+  std::vector<int> node_of_slot;
+  for (int i = 0; i < h->max_nodes; i++) {
+    if (pos[i] < 0 || nodes[i].depth != level + 1 || nodes[i].slot < 0) continue;
+    if (nodes[i].slot >= static_cast<int>(node_of_slot.size())) node_of_slot.resize(nodes[i].slot + 1, -1);
+    node_of_slot[nodes[i].slot] = pos[i];
+  }
+  info->num_slots = static_cast<int32_t>(node_of_slot.size());
+  if (!sum && !hsum && !cnt && !slot_node) return YGG_OK;
+  if (capacity < info->num_slots) return set_error(YGG_ERR_INVALID_ARGUMENT, "capacity %d < %d slots", capacity, info->num_slots);
+  if (hsum && !info->has_hsum) return set_error(YGG_ERR_INVALID_ARGUMENT, "the level has no second histogram plane");
+  if (slot_node) std::copy(node_of_slot.begin(), node_of_slot.end(), slot_node);
+  // the level buffer as k_hist left it, [slot][feature][256] per plane once the chunking is undone
+  const LevelBuf lb = level_buf(h, level_slot_bound(h, level), level == 0 ? 1 : (2 << (level - 1)));
+  std::vector<unsigned long long> buf(lb.total_u64);
+  YGG_CUDA(cudaMemcpy(buf.data(), h->d_capture + h->capture_off[level], lb.total_u64 * sizeof(unsigned long long),
+                      cudaMemcpyDeviceToHost));
+  const unsigned long long* b_sum = buf.data();
+  const unsigned long long* b_hsum = lb.hsum ? buf.data() + (lb.hsum - lb.sum) : nullptr;
+  const uint32_t* b_cnt = reinterpret_cast<const uint32_t*>(buf.data()) + (lb.cnt - reinterpret_cast<uint32_t*>(lb.sum));
+  const int F = info->num_features;
+  for (int s = 0; s < info->num_slots; s++)
+    for (int f = 0; f < F; f++)
+      for (int b = 0; b < kMaxBins; b++) {
+        size_t oc;
+        const size_t o = slot_hist_offset(s, f, b, lb.f_chunk, static_cast<long long>(lb.chunk_u64), &oc);
+        const size_t i = (static_cast<size_t>(s) * F + f) * kMaxBins + b;
+        if (sum) sum[i] = b_sum[o];
+        if (hsum) hsum[i] = b_hsum[o];
+        if (cnt) cnt[i] = b_cnt[oc];
+      }
   return YGG_OK;
 }
 

@@ -135,14 +135,12 @@ __device__ __forceinline__ uint32_t smem_ld_u8(uint32_t addr) {
 
 // Histogram layouts in shared memory (words of 32 bits; B = G*S*256 bins):
 //   kHistShared  : [cnt B][lo B]([hlo B][hhi B])          any S; random bank conflicts (~3.3 wavefronts / ATOMS)
-//   kHistPrivate : [cnt B*32][lo B*32]                    bin (s,b) of lane l at ((s*256+b)*32 + l): every lane
-//                                                         owns a bank => conflict-free atomics; small S only
 //   kHistRootSum : [lo B][carry B]                        shared layout without counts: the root's counts do not
 //                                                         depend on the gradients and are precomputed once
 // Measured on B200 (profiles/atoms_microbench_r01.txt, A/B runs in profiles/k_hist_tuning_r01.md): the
 // shared-memory atomic pipe retires one ATOMS warp-instruction per ~4 cycles per SM whether or not its
-// lanes conflict (up to ~4-way), so bank-conflict-free layouts buy nothing; only the NUMBER of atomic
-// instructions matters.  kHistPrivate is kept for the debug seam and as a measured dead end.
+// lanes conflict (up to ~4-way), so bank-conflict-free layouts (a lane-private copy of every bin was measured) buy
+// nothing; only the NUMBER of atomic instructions matters.
 //   kHistPacked  : [w0 B][w1 B]                            TWO NON-RETURNING atomics (RED) per element and no carry
 //                                                         handling at all: w0 += 1 | (q >> 18) << 13 holds the count
 //                                                         (bits 0..12) and a coarse sum (bits 13..31), w1 += q holds the
@@ -156,7 +154,7 @@ __device__ __forceinline__ uint32_t smem_ld_u8(uint32_t addr) {
 //                                                         kHistShared for levels / datasets where it does not hold.
 // A RED warp-instruction costs ~2.7 clk of the SM's atomic pipe, a returning ATOMS ~5 (tools/atoms_bench.cu), so the
 // packed layout needs 5.4 clk per 32 elements where kHistShared needs 7.7 + the carry fix-ups.
-enum HistMode { kHistShared = 0, kHistPrivate = 1, kHistRootSum = 2, kHistPacked = 3 };
+enum HistMode { kHistShared = 0, kHistRootSum = 1, kHistPacked = 2, kHistModes = 3 };
 constexpr int kPackedCntBits = 13;
 constexpr uint32_t kPackedMaxUpdates = (1u << kPackedCntBits) - 1u;   // 8191 updates of a bin per work item
 constexpr int kPackedCoarseShift = 18;                                // coarse = q >> 18 (6 bits), field 19 bits
@@ -164,8 +162,6 @@ constexpr int kPackedCoarseShift = 18;                                // coarse 
 __host__ __device__ inline size_t hist_bins_bytes(int G, int S, bool hess, int mode) {
   const size_t B = static_cast<size_t>(G) * S * kMaxBins;
   if (mode == kHistShared) return (hess ? 4 : 2) * B * 4;
-  if (mode == kHistPacked) return 2 * B * 4;
-  if (mode == kHistPrivate) return 2 * B * 32 * 4;
   return 2 * B * 4;
 }
 // Shared-memory layout (dynamic):  [histogram][kHistStages x G x 8192 B tiles][mbarriers]
@@ -204,7 +200,7 @@ __global__ void __launch_bounds__(kHistThreads, 1) k_hist(HistParams p) {
   asm volatile("mov.u32 %0, %0;" : "+r"(s_hist));
   const uint32_t hist_bytes = static_cast<uint32_t>(hist_bins_bytes(G, S, HESS, MODE));
   // byte offsets of the planes
-  const uint32_t plane_bytes = static_cast<uint32_t>(B) * 4u * (MODE == kHistPrivate ? 32u : 1u);
+  const uint32_t plane_bytes = static_cast<uint32_t>(B) * 4u;
   const uint32_t s_tiles = s_hist + hist_bytes;
   const uint32_t stage_bytes = static_cast<uint32_t>(G) * kBlockRows;
   const uint32_t s_full = s_tiles + kHistStages * stage_bytes;  // kHistStages full barriers
@@ -234,11 +230,9 @@ __global__ void __launch_bounds__(kHistThreads, 1) k_hist(HistParams p) {
     if constexpr (MULTI) {
       // outside the window: dummy slot
       const uint32_t slot = min((info >> 24) - static_cast<uint32_t>(win_base), static_cast<uint32_t>(S - 1));
-      const uint32_t bin = (slot << 8) | b;
-      return MODE == kHistPrivate ? ((bin << 7) | (lane << 2)) : (bin << 2);
+      return ((slot << 8) | b) << 2;
     } else {
-      const uint32_t bin = ((info >> 24) << 8) | b;
-      return MODE == kHistPrivate ? ((bin << 7) | (lane << 2)) : (bin << 2);
+      return (((info >> 24) << 8) | b) << 2;
     }
   };
 
@@ -399,7 +393,7 @@ __global__ void __launch_bounds__(kHistThreads, 1) k_hist(HistParams p) {
             const bool full = (wb + 31 + (kHistUnroll - 1) * kHistThreads) < n_act;
             if (full) {
               for (int gi = 0; gi < gcount; gi++) {
-                const uint32_t fbase = s_hist + static_cast<uint32_t>(gi * bins_per_feature) * 4u * (MODE == kHistPrivate ? 32u : 1u);
+                const uint32_t fbase = s_hist + static_cast<uint32_t>(gi * bins_per_feature) * 4u;
                 const uint32_t tbase = tile + gi * kBlockRows;
                 uint32_t addr[kHistUnroll], old[kHistUnroll], hold[kHistUnroll];
 #pragma unroll
@@ -439,7 +433,7 @@ __global__ void __launch_bounds__(kHistThreads, 1) k_hist(HistParams p) {
             } else {
               // tail of the block's active list
               for (int gi = 0; gi < gcount; gi++) {
-                const uint32_t fbase = s_hist + static_cast<uint32_t>(gi * bins_per_feature) * 4u * (MODE == kHistPrivate ? 32u : 1u);
+                const uint32_t fbase = s_hist + static_cast<uint32_t>(gi * bins_per_feature) * 4u;
                 const uint32_t tbase = tile + gi * kBlockRows;
 #pragma unroll
                 for (int u = 0; u < kHistUnroll; u++) {
@@ -481,7 +475,7 @@ __global__ void __launch_bounds__(kHistThreads, 1) k_hist(HistParams p) {
       slot_base = win_base;
       used = min(lv.num_slots - slot_base, win_count) * kMaxBins;
     }
-    if (MODE == kHistShared || MODE == kHistRootSum || MODE == kHistPacked) {
+    {
       const uint32_t* s_cnt = hist;              // kHistRootSum: plane 0 = lo, plane 1 = carries
       const uint32_t* s_lo = hist + B;
       const uint32_t* s_hlo = hist + 2 * B;
@@ -522,31 +516,6 @@ __global__ void __launch_bounds__(kHistThreads, 1) k_hist(HistParams p) {
                   s_hlo[gi * bins_per_feature + i];
               atomicAdd(&p.hist_hsum[o], hsum);
             }
-          }
-        }
-      }
-    } else {
-      // lane-private layout: one warp reduces the 32 lane copies of a bin (conflict-free reads).
-      const int warp = tid >> 5;
-      for (int gi = 0; gi < gcount; gi++) {
-        const int f_local = f0 + gi;
-        for (int i = warp; i < used; i += kHistThreads / 32) {
-          const int bin = gi * bins_per_feature + i;
-          const uint32_t c = hist[static_cast<size_t>(bin) * 32 + lane];
-          const uint32_t lo = hist[static_cast<size_t>(B) * 32 + static_cast<size_t>(bin) * 32 + lane];
-          uint32_t cnt = c & ((1u << kHistCntBits) - 1u);
-          unsigned long long sum = (static_cast<unsigned long long>(c >> kHistCntBits) << 32) + lo;
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) {
-            sum += __shfl_xor_sync(0xffffffffu, sum, o);
-            cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-          }
-          if (lane == 0 && cnt != 0u) {
-            const int sl = MULTI ? (i >> 8) + slot_base : (i >> 8), b = i & 0xFF;
-            size_t oc;
-            const size_t o = slot_hist_offset(sl, f_local, b, p.f_chunk, p.chunk_stride, &oc);
-            atomicAdd(&p.hist_sum[o], sum);
-            atomicAdd(&p.hist_cnt[oc], cnt);
           }
         }
       }

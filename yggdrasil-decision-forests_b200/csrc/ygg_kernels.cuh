@@ -35,7 +35,19 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
   return v;
 }
 
-// Power of two P with |g| <= P for all rows, from the float bits of max|g|.
+// Exponent e of the gradient scale P = 2^e: the smallest power of two STRICTLY above max|g| (from its float bits; 1 when
+// every g is 0).  Strictly above, so that g = +max|g| quantises to rint(g * 2^23 / P) + 2^23 < 2^24 instead of being
+// clamped one unit short (the biased 24-bit code has no room for +P).
+__device__ __forceinline__ int pow2_above_exp(unsigned int max_bits) {
+  if (max_bits == 0u) return 0;
+  const int be = static_cast<int>(max_bits >> 23);          // biased exponent; 0: subnormal m * 2^-149
+  return be != 0 ? be - 126 : 32 - __clz(static_cast<int>(max_bits)) - 149;
+}
+// 2^k as a double, k in [-1022, 1023].  The quantisers scale by 2^(23-e), 2^(30-e), 2^(31-2e): for tiny or huge P these
+// leave float range (2^(31-2e) overflows once P <= 2^-49), never double range.
+__device__ __forceinline__ double pow2_d(int k) { return __longlong_as_double(static_cast<long long>(1023 + k) << 52); }
+
+// Power of two P with v <= P, from the float bits of max v (inclusive: the caller's quantiser keeps v = P exact).
 __device__ __forceinline__ float pow2_cover(unsigned int max_bits) {
   if (max_bits == 0u) return 1.f;
   const int e = static_cast<int>(max_bits >> 23) - 127;
@@ -208,26 +220,27 @@ struct QuantParams {
   float hist_h_pow2;       // power of two >= max hist_h
 };
 
-__device__ __forceinline__ uint32_t quant_biased(float v, float scale, uint32_t bias, uint32_t vmax) {
+__device__ __forceinline__ uint32_t quant_biased(float v, double scale, uint32_t bias, uint32_t vmax) {
   // rint(v * scale) + bias, clamped to [0, vmax]; scale is a power of two so v*scale is exact.
-  const float t = rintf(v * scale) + static_cast<float>(bias);
-  return static_cast<uint32_t>(fminf(fmaxf(t, 0.f), static_cast<float>(vmax)));
+  const double t = rint(static_cast<double>(v) * scale) + static_cast<double>(bias);
+  return static_cast<uint32_t>(fmin(fmax(t, 0.0), static_cast<double>(vmax)));
 }
-// 31-bit statistics quantisers.  `scale` is a power of two, so v*scale is exact in float; the
-// conversion rounds to the nearest integer (values >= 2^24 are already integers).  Saturating.
-__device__ __forceinline__ uint32_t quant_stat_signed(float v, float scale) {   // -> [0, 2^31], bias 2^30
-  const int t = __float2int_rn(v * scale);                                       // |v*scale| <= 2^30
+// 31-bit statistics quantisers.  `scale` is a power of two, so v*scale is exact; the conversion rounds to the nearest
+// integer.  Saturating.  (A float scale gives the same results wherever it is finite: the product is exact either way.)
+__device__ __forceinline__ uint32_t quant_stat_signed(float v, double scale) {   // -> [0, 2^31], bias 2^30
+  const int t = __double2int_rn(static_cast<double>(v) * scale);                 // |v*scale| <= 2^30
   return static_cast<uint32_t>(min(max(t, -(1 << 30)), (1 << 30)) + (1 << 30));
 }
-__device__ __forceinline__ uint32_t quant_stat_unsigned(float v, float scale) {  // v >= 0 -> [0, 2^31]
-  return min(__float2uint_rn(v * scale), 0x80000000u);  // v == its power-of-two cover stays exact
+__device__ __forceinline__ uint32_t quant_stat_unsigned(float v, double scale) {  // v >= 0 -> [0, 2^31]
+  return min(__double2uint_rn(static_cast<double>(v) * scale), 0x80000000u);  // v == its power-of-two cover stays exact
 }
 
 __global__ void __launch_bounds__(256) k_quantize(QuantParams p) {
-  const float P = p.fixed_g_pow2 > 0.f ? p.fixed_g_pow2 : pow2_cover(p.st->gmax_bits);
-  const float qscale = static_cast<float>(1u << (kQBits - 1)) / P;     // 2^23 / P
-  const float sscale = static_cast<float>(1u << (kSBits - 1)) / P;     // 2^30 / P
-  const float s2scale = static_cast<float>(1u << kSBits) / (P * P);    // g^2 in [0, P^2]
+  const int e = p.fixed_g_pow2 > 0.f ? ilogbf(p.fixed_g_pow2) : pow2_above_exp(p.st->gmax_bits);   // P = 2^e
+  const float P = ldexpf(1.f, e);
+  const double qscale = pow2_d(kQBits - 1 - e);    // 2^23 / P
+  const double sscale = pow2_d(kSBits - 1 - e);    // 2^30 / P
+  const double s2scale = pow2_d(kSBits - 2 * e);   // g^2 in [0, P^2]
   const float hscale = static_cast<float>(1u << kSBits) / p.h_pow2;    // h in [0, h_pow2]
   const float hqscale = static_cast<float>(1u << kQBits) / (p.hist_h != nullptr ? p.hist_h_pow2 : p.h_pow2);
   unsigned long long sg = 0, sh = 0, sg2 = 0;
@@ -1101,9 +1114,9 @@ __global__ void __launch_bounds__(kPartThreads, 2) k_partition(PartParams p) {
     }
   }
   __syncthreads();
-  const float P = p.st->g_pow2;
-  const float sscale = static_cast<float>(1u << (kSBits - 1)) / P;
-  const float s2scale = static_cast<float>(1u << kSBits) / (P * P);
+  const int e = ilogbf(p.st->g_pow2);             // P = 2^e, see k_quantize
+  const double sscale = pow2_d(kSBits - 1 - e);
+  const double s2scale = pow2_d(kSBits - 2 * e);
   const float hscale = static_cast<float>(1u << kSBits) / p.st->h_pow2;
   for (int blk = blockIdx.x; blk < p.n_blocks; blk += gridDim.x) {
     const int64_t base = static_cast<int64_t>(blk) * kBlockRows;
