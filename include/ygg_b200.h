@@ -364,17 +364,16 @@ enum ygg_hist_layout {
   YGG_HIST_LAYOUT_SHARED_HESS = 3,        /* YGG_HIST_LAYOUT_SHARED + the second plane (hessians or weights) */
   YGG_HIST_LAYOUT_PACKED_MULTI = 4,       /* the windowed instantiations: `passes` launches over windows of slots */
   YGG_HIST_LAYOUT_SHARED_MULTI = 5,
-  YGG_HIST_LAYOUT_SHARED_HESS_MULTI = 6,
-  YGG_HIST_LAYOUT_HIST2 = 7               /* k_hist2 with `hist2_lanes` feature lanes */
+  YGG_HIST_LAYOUT_SHARED_HESS_MULTI = 6
 };
 
 typedef struct ygg_hist_level_info {
   int32_t layout;             /* enum ygg_hist_layout */
-  int32_t features_per_item;  /* k_hist: G features per work item (0 for k_hist2) */
+  int32_t features_per_item;  /* k_hist: G features per work item */
   int32_t smem_slots;         /* k_hist: slots in shared memory (windowed: window + 1 dummy slot) */
   int32_t passes;             /* launches of the level (> 1: windowed) */
   int32_t chunk_blocks;       /* 8192-row blocks per work item */
-  int32_t hist2_lanes;        /* k_hist2 feature lanes, 0 for k_hist */
+  int32_t reserved;           /* always 0 */
   int32_t num_slots;          /* histogram slots of the level */
   int32_t feature_begin;      /* histogrammed features of this rank: [feature_begin, feature_begin + num_features) */
   int32_t num_features;

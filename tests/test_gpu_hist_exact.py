@@ -6,8 +6,8 @@ every row through the returned tree, and bincount q, hq and the counts per (slot
 cannot see a wrong bin unless it changes which split wins; this file compares the planes themselves, as the level
 loop computed them (ygg_gbt_debug_capture_histograms), for every layout configure_launches can pick: the root's carry
 plane, the packed words on both sides of their bound, the carry-detecting fallback with and without the hessian
-planes, the windowed deep levels, k_hist2, sampled and weighted roots and row shards.  Each case asserts the layout
-it expects, so that a case cannot silently stop covering the path it names.
+planes, the windowed deep levels, sampled and weighted roots and row shards.  Each case asserts the layout it expects,
+so that a case cannot silently stop covering the path it names.
 """
 import numpy as np
 import pytest
@@ -56,8 +56,10 @@ def test_root_sum_row_count_edges(n, monkeypatch):
 
 # ---- packed words: partial feature groups, edge bin counts, categorical columns ----------------------------------
 
-@pytest.mark.parametrize("F", [1, 7, 9])
-def test_packed_feature_groups_and_bins(F):
+def _packed_case(F):
+    """F columns of 256, 2 and 255 bins, the last bin of each populated, every 4th column categorical: one tree of
+    depth 5 on them.  Returns (bins, nbs, tree, captures of its 4 levels, which must be root_sum, packed, packed,
+    packed)."""
     n = 50000
     rng = np.random.default_rng(F)
     nbs = [(256, 2, 255)[j % 3] for j in range(F)]
@@ -68,10 +70,30 @@ def test_packed_feature_groups_and_bins(F):
     ds, gbt = _gbt(bins, np.array(nbs, np.int32), np.zeros(F, np.int32), ft=ft, loss=1, max_depth=5)
     g = _grad(bins, F)
     tree = gbt.train_tree_on_gradients(g)
-    assert len(tree) > 7
     caps = check_levels(gbt, tree, bins, ["root_sum"] + ["packed"] * 3)
+    return bins, nbs, tree, caps
+
+
+@pytest.mark.parametrize("F", [1, 7, 9])
+def test_packed_feature_groups_and_bins(F):
+    bins, nbs, tree, caps = _packed_case(F)
+    assert len(tree) > 7
     for j, k in enumerate(nbs):
         assert caps[0]["cnt"][0, j, k - 1] >= 50
+
+
+def test_retired_switches_are_ignored(monkeypatch):
+    """The layout of every level follows from the configuration alone: the environment switches that once selected
+    the feature-lane kernel (YGG_HIST2) or turned the root's and the packed layouts off change nothing."""
+    def run():
+        _, _, tree, caps = _packed_case(9)
+        return tree.tobytes(), [(c["chunk_blocks"], c["features_per_item"], c["smem_slots"]) for c in caps]
+
+    base = run()
+    monkeypatch.setenv("YGG_HIST2", "1")
+    monkeypatch.setenv("YGG_HIST_ROOT_SUM", "0")
+    monkeypatch.setenv("YGG_HIST_PACKED", "0")
+    assert run() == base
 
 
 @pytest.mark.parametrize("heavy", [8191, 8192])
@@ -168,19 +190,6 @@ def test_multi_window_levels(depth, hess):
     assert multi and all(c["passes"] > 1 for c in multi)
     assert multi[-1]["layout"] == ("shared_hess_multi" if hess else "packed_multi")
     assert max(c["num_slots"] for c in multi) > multi[-1]["smem_slots"]   # the windows really split the slots
-
-
-# ---- k_hist2 -------------------------------------------------------------------------------------------------------
-
-@pytest.mark.parametrize("F,FL", [(4, 8), (9, 16), (40, 32)])
-def test_hist2_feature_lanes(F, FL, monkeypatch):
-    monkeypatch.setenv("YGG_HIST2", "1")
-    n = 60000
-    bins, nb, na, _ = synth(n, F, seed=F, bins=255)
-    ds, gbt = _gbt(bins, nb, na, loss=1, max_depth=5)
-    tree = gbt.train_tree_on_gradients(_grad(bins, F))
-    caps = check_levels(gbt, tree, bins, ["hist2", "hist2", "hist2", None])
-    assert all(c["hist2_lanes"] == FL for c in caps[:3])
 
 
 # ---- sampled roots, GOSS, example weights --------------------------------------------------------------------------

@@ -256,27 +256,6 @@ def test_reference_label_classes_order(label_data):
     assert model.num_trees() == 1
 
 
-def test_feature_lane_histogram_kernel_is_bit_identical(monkeypatch):
-    """k_hist2 (csrc/ygg_hist2.cuh: lanes = features, [bin][feature] histograms, interleaved copy of the matrix) is an
-    alternative to k_hist on the levels with <= 2 slots; integer sums make the two bit-identical.  Off by default
-    (it is not faster, DESIGN.md §5); YGG_HIST2=1 turns it on for handles created afterwards."""
-    bins, nb, na, y = synth(60000, 40, seed=11, bins=255)
-
-    def run():
-        ds = ydf_b200.Dataset(bins, nb, na)
-        gbt = ydf_b200.Gbt(ds, ydf_b200.default_config(max_depth=6, num_trees=4))
-        gbt.set_labels(y)
-        gbt.train(4)
-        out = [gbt.get_tree(i).tobytes() for i in range(4)], [gbt.train_loss(i) for i in range(4)]
-        gbt.close()
-        ds.close()
-        return out
-
-    base = run()
-    monkeypatch.setenv("YGG_HIST2", "1")
-    assert run() == base
-
-
 @pytest.mark.parametrize("mode,threads", [(2, 4), (1, 4)])
 def test_tie_break_follows_the_candidate_shuffle(mode, threads):
     """a5: between features whose best splits have EQUAL float scores the reference takes the first in the order of

@@ -44,13 +44,13 @@ FEATURE_DISCRETIZED_NUMERICAL = 0
 FEATURE_CATEGORICAL = 1
 
 # enum ygg_hist_layout
-HIST_LAYOUTS = ("root_sum", "packed", "shared", "shared_hess", "packed_multi", "shared_multi", "shared_hess_multi", "hist2")
+HIST_LAYOUTS = ("root_sum", "packed", "shared", "shared_hess", "packed_multi", "shared_multi", "shared_hess_multi")
 
 
 class HistLevelInfo(C.Structure):
     _fields_ = [
         ("layout", C.c_int32), ("features_per_item", C.c_int32), ("smem_slots", C.c_int32), ("passes", C.c_int32),
-        ("chunk_blocks", C.c_int32), ("hist2_lanes", C.c_int32), ("num_slots", C.c_int32), ("feature_begin", C.c_int32),
+        ("chunk_blocks", C.c_int32), ("reserved", C.c_int32), ("num_slots", C.c_int32), ("feature_begin", C.c_int32),
         ("num_features", C.c_int32), ("has_hsum", C.c_int32), ("g_pow2", C.c_float), ("h2_pow2", C.c_float),
         ("n_rows", C.c_int64), ("g", C.POINTER(C.c_float)), ("h2", C.POINTER(C.c_float)), ("selected", C.POINTER(C.c_uint8)),
     ]

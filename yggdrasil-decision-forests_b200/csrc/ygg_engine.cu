@@ -121,8 +121,19 @@ struct LossRec {
 
 enum ShardMode { kShardNone = 0, kShardFeatures = 1, kShardRows = 2 };
 
+// k_hist launches of one tree level: num_sms persistent CTAs of the instantiation for (mode, hessian planes, passes > 1).
+struct HistLevel {
+  int mode;           // kHistRootSum / kHistPacked / kHistShared (ygg_hist.cuh)
+  int G;              // features per work item
+  int S;              // slots in shared memory (windowed: window + 1 dummy slot)
+  int passes;         // > 1: the level's slots are accumulated in windows of S - 1 slots, one launch each
+  int chunk_blocks;   // 8192-row blocks per work item
+  size_t smem;        // dynamic shared memory per CTA
+};
+
 struct ygg_gbt {
   ygg_dataset* ds = nullptr;
+  int device = 0;   // ds->device: ygg_gbt_destroy must not read `ds`, which may already be destroyed
   ygg_gbt_config cfg{};
   cudaStream_t stream = nullptr;
   bool has_labels = false;
@@ -137,7 +148,6 @@ struct ygg_gbt {
   uint2* d_act = nullptr;
   uint32_t* d_act_h = nullptr;
   int32_t* d_act_count = nullptr;
-  int32_t* d_act_sub = nullptr;    // [n_blocks][8], see PartParams
   uint32_t* d_root_cnt = nullptr;  // [f_count][256] row counts of the root (gradient independent)
   bool root_cnt_valid = false;
   int n_blocks = 0;
@@ -228,11 +238,8 @@ struct ygg_gbt {
   void* exchange_ctx = nullptr;
   void** d_peer_windows = nullptr;   // [world] best-split windows of every rank as mapped in this process (or null)
   uint32_t exchange_epoch = 0;
-  // launch configuration
-  int hist_grid[32]{}, hist_G[32]{}, hist_S[32]{}, hist_chunk[32]{}, hist_mode[32]{};
-  int hist_passes[32]{};               // > 1: the level's slots are accumulated in windows of hist_S[l] - 1 slots (k_hist<.., MULTI>)
-  int hist2_FL[32]{}, hist2_T[32]{};   // > 0: the level runs k_hist2 with FL feature lanes and T sub-tiles per tile
-  size_t hist_smem[32]{};
+  // launch configuration (configure_launches)
+  HistLevel hist[32]{};
   int part_smem_children = 0;
   // histogram capture (ygg_gbt_debug_capture_histograms): every level's slot planes of the last tree grown
   bool capture_hist = false;
@@ -436,81 +443,45 @@ int chunk_max_count(ygg_gbt* h, int chunk_blocks, uint32_t** d_sub, uint32_t* ou
   return YGG_OK;
 }
 
+// cudaFuncAttributeMaxDynamicSharedMemorySize is a per-kernel cap of the current device, shared by every handle of the
+// process (handles with other feature shards, or on other devices, may coexist): raise it to the full budget on every
+// k_hist instantiation.  It is only a cap: each launch asks for its level's HistLevel::smem.
+int raise_hist_smem_cap(size_t budget) {
+  auto cap = [&](auto kern) -> int {
+    YGG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(budget)));
+    return YGG_OK;
+  };
+  YGG_RETURN_IF_ERROR(cap(k_hist<false, kHistRootSum>));
+  YGG_RETURN_IF_ERROR(cap(k_hist<false, kHistPacked>));
+  YGG_RETURN_IF_ERROR(cap(k_hist<false, kHistShared>));
+  YGG_RETURN_IF_ERROR(cap(k_hist<true, kHistShared>));
+  YGG_RETURN_IF_ERROR(cap(k_hist<false, kHistPacked, true>));
+  YGG_RETURN_IF_ERROR(cap(k_hist<false, kHistShared, true>));
+  return cap(k_hist<true, kHistShared, true>);
+}
+
+// The k_hist launches of every level (HistLevel).  Layout: with the hessian or weight planes, kHistShared; at an
+// unsampled root, kHistRootSum (the root's counts are gradient independent and precomputed: no count atomics); else
+// kHistPacked (two REDs per element instead of a RED and a returning ATOMS), which falls back to kHistShared when a bin
+// could receive more than kPackedMaxUpdates updates inside one work item.
 int configure_launches(ygg_gbt* h) {
   const bool hh = hist_hess(h);
   const size_t budget = 224 * 1024;  // dynamic shared memory per CTA we are willing to use (227 KB max)
   const int f_count = h->hist_f_end - h->hist_f_begin;  // features histogrammed by this rank
-  for (int l = 0; l < h->num_levels; l++) {
-    // Lane-private (bank-conflict-free) layouts while they fit; the root additionally skips the
-    // count atomics (precomputed counts).
-    // The root skips the count atomics (its counts are gradient independent and precomputed).
-    // YGG_HIST_ROOT_SUM=0 disables that (tuning / A-B knob).
-    int mode = kHistShared;
-    if (!hh && l == 0 && !sampling(h)) {   // (a sampled root is not the whole dataset: its counts are not the precomputed ones)
-      const char* env = std::getenv("YGG_HIST_ROOT_SUM");
-      if (!env || std::atoi(env) != 0) mode = kHistRootSum;
-    }
-    if (!hh && (l > 0 || sampling(h))) {
-      // two REDs per element instead of RED + returning ATOMS; confirmed (or taken back) below, once the chunk
-      // sizes are known: no bin may receive more than 8191 updates inside one work item.  YGG_HIST_PACKED=0: A/B knob.
-      const char* env = std::getenv("YGG_HIST_PACKED");
-      if (!env || std::atoi(env) != 0) mode = kHistPacked;
-    }
-    int S = level_slot_bound(h, l);
-    h->hist_passes[l] = 1;
-    if (hist_smem_bytes(1, S, hh, mode) > budget) {
-      // more slots than shared memory holds: windows of S_pass slots (+ 1 dummy slot for the rows of the other windows),
-      // one launch per window.  The slot of a row travels in 8 bits of its active-list entry (0xFF = none).
-      if (S > 254)
-        return set_error(YGG_ERR_UNIMPLEMENTED, "max_depth=%d needs %d histogram slots at level %d; the active lists carry 8-bit slots",
-                         h->cfg.max_depth, S, l);
-      int s_pass = 1;
-      while (hist_smem_bytes(1, 2 * s_pass + 1, hh, mode) <= budget) s_pass *= 2;
-      h->hist_passes[l] = (S + s_pass - 1) / s_pass;
-      S = s_pass + 1;
-    }
-    int G = 1;
-    while (G < 8 && G < f_count && hist_smem_bytes(G + 1, S, hh, mode) <= budget) G++;
-    h->hist_G[l] = G;
-    h->hist_S[l] = S;
-    h->hist_mode[l] = mode;
-    h->hist_smem[l] = hist_smem_bytes(G, S, hh, mode);
-  }
-  for (int mode = 0; mode < kHistModes; mode++) {
-    size_t max_smem = 0;
-    for (int l = 0; l < h->num_levels; l++)
-      if (h->hist_mode[l] == mode) max_smem = std::max(max_smem, h->hist_smem[l]);
-    if (mode == kHistPacked && !hh) max_smem = std::max<size_t>(max_smem, 1);  // a level may fall back to / from it
-    if (mode == kHistShared && !hh) max_smem = std::max<size_t>(max_smem, 1);
-    if (max_smem == 0) continue;
-    // The attribute is a per-kernel cap shared by every handle of the process (several handles with
-    // different feature shards may coexist): always raise it to the full budget.
-    const int st = for_hist_kernel(hh, mode, [&](auto kern) -> int {
-      YGG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(budget)));
-      return YGG_OK;
-    });
-    if (st != YGG_OK) return st;
-    if (hh) break;
-  }
   const int n_blocks = static_cast<int>(h->ds->n_pad / kBlockRows);
+  const int grid = h->ds->num_sms;
   const int kSubBlocks = sub_blocks_of(h);
-  static const double min_items = [] {   // tuning knob (default 3 work items per CTA)
-    const char* v = std::getenv("YGG_HIST_ITEMS_PER_CTA");
-    return v ? std::atof(v) : 1.0;   // measured: whole waves beat many small items on C2, C3 and at 1.25M rows per rank
-  }();
-  // Row blocks per work item (a multiple of `step`): as many as the bin counters allow (the flush to the global
-  // histogram is amortised over the chunk), but few enough that every CTA gets >= min_items items, and among those
-  // the size whose item count fills whole waves of the persistent grid (static round-robin over CTAs).
-  static const double min_items2 = [] {   // k_hist2 levels: few, equal items (default: one wave)
-    const char* v = std::getenv("YGG_HIST2_ITEMS_PER_CTA");
-    return v ? std::atof(v) : 0.9;
-  }();
+  // Row blocks per work item of G features (a multiple of `step`): as many as the bin counters allow (the flush to the
+  // global histogram is amortised over the chunk), but few enough that every CTA gets at least one item, and among
+  // those the size whose item count fills whole waves of the persistent grid (static round-robin over CTAs; measured:
+  // whole waves beat many small items on C2, C3 and at 1.25M rows per rank).
   // YGG_HIST_CHUNK_BLOCKS=c (tests: reach the chunk sizes where the bin counters come closest to their limits) forces
   // c row blocks per work item, clamped to [step, kHistMaxChunkBlocks] and rounded down to the step.  Read at every
-  // configure, like YGG_HIST2.
+  // configure.
   const char* env_chunk = std::getenv("YGG_HIST_CHUNK_BLOCKS");
   const int forced_chunk = env_chunk != nullptr ? std::atoi(env_chunk) : 0;
-  auto choose_chunk = [&](int n_fgroups, int grid, int step, double need) {
+  auto choose_chunk = [&](int G, int step) {
+    const int n_fgroups = (f_count + G - 1) / G;
     const int max_c = std::max(step, kHistMaxChunkBlocks / step * step);
     if (forced_chunk > 0) return std::max(step, std::min(forced_chunk, max_c) / step * step);
     const int min_chunks = std::max(1, (n_blocks + max_c - 1) / max_c);
@@ -525,46 +496,45 @@ int configure_launches(ygg_gbt* h) {
       // a short last chunk leaves its CTAs idle for the rest of a round: weigh the waves by the rows they carry
       const double fill = static_cast<double>(n_blocks) / (static_cast<double>(real_nc) * c);
       const double eff = per_cta / std::ceil(per_cta) * fill;
-      // whole waves first (an unfilled last wave idles the GPU), then enough items per CTA to even out their durations
-      const double score = eff + (per_cta >= need ? 0.08 : 0.0);
+      // whole waves first (an unfilled last wave idles the GPU), then at least one item per CTA
+      const double score = eff + (per_cta >= 1.0 ? 0.08 : 0.0);
       if (score > best_score + 1e-9) { best_score = score; best = c; }
     }
     return best;
   };
-  // k_hist2 (feature-per-lane, bank-conflict-free; ygg_hist2.cuh) on the shallow levels.  OFF by default: measured on
-  // C3 it ties k_hist at the root (1.03 ms) and at level 1 and loses at level 2 (DESIGN.md §5, profiles/k_hist2_r02.md),
-  // while costing a second copy of the matrix.  YGG_HIST2=1 enables it (read at every configure: tests toggle it).
-  const int g_begin = h->hist_f_begin / 4, n_groups = (h->hist_f_end + 3) / 4 - g_begin;
-  const size_t budget2 = 216 * 1024;   // k_hist2 also holds 4.6 KB of static shared memory (sub-tile offsets)
-  const char* env_hist2 = std::getenv("YGG_HIST2");
-  const bool want_hist2 = env_hist2 != nullptr && std::atoi(env_hist2) != 0;
   for (int l = 0; l < h->num_levels; l++) {
-    h->hist_grid[l] = h->ds->num_sms;  // persistent: one CTA per SM
-    h->hist2_FL[l] = 0;
-    const int S = h->hist_S[l];
-    // S <= 2: 32 feature lanes fit; at S = 4 only 16 would (two rows per instruction: bank conflicts come back and the
-    // gain over k_hist is gone: tools/hist_loop_bench.cu)
-    if (want_hist2 && !hh && S <= 2 && (l > 0 || h->hist_mode[0] == kHistRootSum)) {
-      int FL = 32;
-      while (FL > 8 && FL / 2 >= 4 * n_groups) FL /= 2;   // few features: no idle lanes
-      int T = 2;
-      if (hist2_smem_bytes(FL, S, T, l == 0) > budget2) T = 1;
-      if (hist2_smem_bytes(FL, S, T, l == 0) <= budget2) { h->hist2_FL[l] = FL; h->hist2_T[l] = T; }
+    HistLevel& hl = h->hist[l];
+    // (a sampled root is not the whole dataset: its counts are not the precomputed ones)
+    hl.mode = hh ? kHistShared : (l == 0 && !sampling(h)) ? kHistRootSum : kHistPacked;
+    int S = level_slot_bound(h, l);
+    hl.passes = 1;
+    if (hist_smem_bytes(1, S, hh, hl.mode) > budget) {
+      // more slots than shared memory holds: windows of S_pass slots (+ 1 dummy slot for the rows of the other windows),
+      // one launch per window.  The slot of a row travels in 8 bits of its active-list entry (0xFF = none).
+      if (S > 254)
+        return set_error(YGG_ERR_UNIMPLEMENTED, "max_depth=%d needs %d histogram slots at level %d; the active lists carry 8-bit slots",
+                         h->cfg.max_depth, S, l);
+      int s_pass = 1;
+      while (hist_smem_bytes(1, 2 * s_pass + 1, hh, hl.mode) <= budget) s_pass *= 2;
+      hl.passes = (S + s_pass - 1) / s_pass;
+      S = s_pass + 1;
     }
-    const bool packed = h->hist_mode[l] == kHistPacked || (h->hist2_FL[l] > 0 && l > 0);   // (k_hist2 is not used at a sampled root: hist_mode[0] != kHistRootSum)
-    const int n_fgroups = h->hist2_FL[l] > 0 ? (n_groups + h->hist2_FL[l] / 4 - 1) / (h->hist2_FL[l] / 4)
-                                              : (f_count + h->hist_G[l] - 1) / h->hist_G[l];
-    h->hist_chunk[l] = choose_chunk(n_fgroups, h->hist_grid[l], packed ? kSubBlocks : 1, h->hist2_FL[l] > 0 ? min_items2 : min_items);
+    int G = 1;
+    while (G < 8 && G < f_count && hist_smem_bytes(G + 1, S, hh, hl.mode) <= budget) G++;
+    hl.G = G;
+    hl.S = S;
+    hl.smem = hist_smem_bytes(G, S, hh, hl.mode);
+    hl.chunk_blocks = choose_chunk(G, hl.mode == kHistPacked ? kSubBlocks : 1);
   }
-  // Packed words (kHistPacked and k_hist2 below the root): the dataset-level bound on the updates a bin can receive
-  // inside one work item (ygg_hist.cuh).
+  // The packed words' bound: the dataset-level largest count a bin can receive inside one work item (ygg_hist.cuh).
   {
     std::map<int, uint32_t> max_of_chunk;   // chunk size -> largest per-bin count of any (chunk, feature)
     uint32_t* d_sub = nullptr;
     int status = YGG_OK;
     for (int l = 0; l < h->num_levels && status == YGG_OK; l++) {
-      if (h->hist_mode[l] != kHistPacked && (h->hist2_FL[l] == 0 || l == 0)) continue;
-      int chunk = h->hist_chunk[l];
+      HistLevel& hl = h->hist[l];
+      if (hl.mode != kHistPacked) continue;
+      int chunk = hl.chunk_blocks;
       while (chunk >= kSubBlocks) {
         auto it = max_of_chunk.find(chunk);
         if (it == max_of_chunk.end()) {
@@ -579,41 +549,16 @@ int configure_launches(ygg_gbt* h) {
         chunk = std::min(smaller, chunk - kSubBlocks);
       }
       if (chunk < kSubBlocks) {   // heavy bins (a dominant value / category): the carry-detecting layout, any chunk size
-        h->hist_mode[l] = kHistShared;
-        h->hist2_FL[l] = 0;
-        h->hist_chunk[l] = choose_chunk((f_count + h->hist_G[l] - 1) / h->hist_G[l], h->hist_grid[l], 1, min_items);
+        hl.mode = kHistShared;    // (the same shared memory as kHistPacked without the hessian planes)
+        hl.chunk_blocks = choose_chunk(hl.G, 1);
       } else {
-        h->hist_chunk[l] = chunk;
+        hl.chunk_blocks = chunk;
       }
     }
     dev_free(d_sub);
     if (status != YGG_OK) return status;
   }
-  {
-    auto set_attr = [&](auto kern) -> int {
-      YGG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(budget2)));
-      return YGG_OK;
-    };
-    bool any_multi = false;
-    for (int l = 0; l < h->num_levels; l++) any_multi |= h->hist_passes[l] > 1;
-    if (any_multi) {
-      const int st = for_hist_kernel(hh, kHistPacked, [&](auto kern) -> int {
-        YGG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(budget)));
-        return YGG_OK;
-      }, true);
-      if (st != YGG_OK) return st;
-      if (!hh) {
-        const int st2 = for_hist_kernel(false, kHistShared, [&](auto kern) -> int {
-          YGG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(budget)));
-          return YGG_OK;
-        }, true);
-        if (st2 != YGG_OK) return st2;
-      }
-    }
-    YGG_RETURN_IF_ERROR(set_attr(k_hist2<32, true>)); YGG_RETURN_IF_ERROR(set_attr(k_hist2<32, false>));
-    YGG_RETURN_IF_ERROR(set_attr(k_hist2<16, true>)); YGG_RETURN_IF_ERROR(set_attr(k_hist2<16, false>));
-    YGG_RETURN_IF_ERROR(set_attr(k_hist2<8, true>)); YGG_RETURN_IF_ERROR(set_attr(k_hist2<8, false>));
-  }
+  YGG_RETURN_IF_ERROR(raise_hist_smem_cap(budget));
   // k_partition shared accumulators: up to 32 KB (one copy) / 14 KB (lane-private, <= 16 children).
   h->part_smem_children = static_cast<int>((32 * 1024) / (kPartWords * sizeof(uint32_t)));
   return YGG_OK;
@@ -653,36 +598,12 @@ int allocate_level_buffers(ygg_gbt* h) {
   return YGG_OK;
 }
 
-int launch_hist(ygg_gbt* h, const HistParams& hp, int mode, int grid, size_t smem, bool multi = false) {
-  return for_hist_kernel(hist_hess(h), mode, [&](auto kern) -> int {
-    kern<<<grid, kHistThreads, smem, h->stream>>>(hp);
+int launch_hist(ygg_gbt* h, const HistParams& hp, const HistLevel& hl) {
+  return for_hist_kernel(hist_hess(h), hl.mode, [&](auto kern) -> int {
+    kern<<<h->ds->num_sms, kHistThreads, hl.smem, h->stream>>>(hp);   // persistent: one CTA per SM
     h->launches_total++;
     return check_launch("k_hist");
-  }, multi);
-}
-
-// The interleaved copy of the matrix k_hist2 reads (ygg_hist2.cuh), built on first use and kept with the dataset.
-int ensure_bins4(ygg_dataset* ds) {
-  if (ds->d_bins4 != nullptr) return YGG_OK;
-  const int groups = (ds->F + 3) / 4;
-  YGG_RETURN_IF_ERROR(dev_alloc(&ds->d_bins4, static_cast<size_t>(groups) * ds->n_pad));
-  dim3 grid(static_cast<unsigned>(std::min<int64_t>((ds->n_pad / 4 + 255) / 256, 4096)), static_cast<unsigned>(groups));
-  k_interleave4<<<grid, 256>>>(ds->d_bins, ds->n_pad, ds->F, ds->d_bins4);
-  YGG_RETURN_IF_ERROR(check_launch("k_interleave4"));
-  YGG_CUDA(cudaDeviceSynchronize());
-  return YGG_OK;
-}
-
-int launch_hist2(ygg_gbt* h, const Hist2Params& hp, int FL, bool root, int grid) {
-  const size_t smem = hist2_smem_bytes(FL, hp.S, hp.T, root);
-  auto go = [&](auto kern) -> int {
-    kern<<<grid, kHist2Threads, smem, h->stream>>>(hp);
-    h->launches_total++;
-    return check_launch("k_hist2");
-  };
-  if (FL == 32) return root ? go(k_hist2<32, true>) : go(k_hist2<32, false>);
-  if (FL == 16) return root ? go(k_hist2<16, true>) : go(k_hist2<16, false>);
-  return root ? go(k_hist2<8, true>) : go(k_hist2<8, false>);
+  }, hl.passes > 1);
 }
 
 // Root count histogram: once per (dataset, shard).
@@ -730,6 +651,15 @@ int launch_weight_sums(ygg_gbt* h, NodeRec* nodes) {
   return check_launch("k_weight_sums");
 }
 
+// The enum ygg_hist_layout value of a level's launches (the k_hist instantiation for_hist_kernel picks).
+int hist_layout(const HistLevel& hl, bool hess) {
+  const bool multi = hl.passes > 1;
+  if (hess) return multi ? YGG_HIST_LAYOUT_SHARED_HESS_MULTI : YGG_HIST_LAYOUT_SHARED_HESS;
+  if (hl.mode == kHistRootSum) return YGG_HIST_LAYOUT_ROOT_SUM;
+  if (hl.mode == kHistPacked) return multi ? YGG_HIST_LAYOUT_PACKED_MULTI : YGG_HIST_LAYOUT_PACKED;
+  return multi ? YGG_HIST_LAYOUT_SHARED_MULTI : YGG_HIST_LAYOUT_SHARED;
+}
+
 // Histogram capture: sizes the buffers for this handle's level geometry and records the launch configuration of every
 // level and the quantiser's float inputs `q` of the tree about to be grown.
 int begin_capture(ygg_gbt* h, const QuantParams& q) {
@@ -766,17 +696,12 @@ int begin_capture(ygg_gbt* h, const QuantParams& q) {
   const bool hess = hist_hess(h);
   for (int l = 0; l < h->num_levels; l++) {
     ygg_hist_level_info& in = h->capture_info[l];
-    const bool multi = h->hist_passes[l] > 1;
-    if (h->hist2_FL[l] > 0) in.layout = YGG_HIST_LAYOUT_HIST2;
-    else if (hess) in.layout = multi ? YGG_HIST_LAYOUT_SHARED_HESS_MULTI : YGG_HIST_LAYOUT_SHARED_HESS;
-    else if (h->hist_mode[l] == kHistRootSum) in.layout = YGG_HIST_LAYOUT_ROOT_SUM;
-    else if (h->hist_mode[l] == kHistPacked) in.layout = multi ? YGG_HIST_LAYOUT_PACKED_MULTI : YGG_HIST_LAYOUT_PACKED;
-    else in.layout = multi ? YGG_HIST_LAYOUT_SHARED_MULTI : YGG_HIST_LAYOUT_SHARED;
-    in.features_per_item = h->hist2_FL[l] > 0 ? 0 : h->hist_G[l];
-    in.smem_slots = h->hist_S[l];
-    in.passes = h->hist_passes[l];
-    in.chunk_blocks = h->hist_chunk[l];
-    in.hist2_lanes = h->hist2_FL[l];
+    const HistLevel& hl = h->hist[l];
+    in.layout = hist_layout(hl, hess);
+    in.features_per_item = hl.G;
+    in.smem_slots = hl.S;
+    in.passes = hl.passes;
+    in.chunk_blocks = hl.chunk_blocks;
     in.feature_begin = h->hist_f_begin;
     in.num_features = h->hist_f_end - h->hist_f_begin;
     in.has_hsum = hess ? 1 : 0;
@@ -800,7 +725,7 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
   const bool rows_sharded = h->shard_mode == kShardRows;
   const int64_t n_job = sampling(h) ? h->n_selected : (rows_sharded ? h->n_global : ds->n);   // rows the tree is trained on
   const int root_candidate = (n_job >= h->cfg.min_examples && 1 < h->cfg.max_depth) ? 1 : 0;
-  if (h->num_levels > 0 && h->hist_mode[0] == kHistRootSum) YGG_RETURN_IF_ERROR(ensure_root_counts(h));
+  if (h->num_levels > 0 && h->hist[0].mode == kHistRootSum) YGG_RETURN_IF_ERROR(ensure_root_counts(h));
   const bool hess = hist_hess(h);
   auto slots_of = [&](int l) { return level_slot_bound(h, l); };
   {
@@ -824,7 +749,7 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
     YGG_RETURN_IF_ERROR(check_launch("k_quantize"));
     if (sampling(h)) {   // the root's active lists = the sampled rows
       k_compact_root<<<std::min(h->n_blocks, h->ds->num_sms * 4), kCompactThreads, 0, h->stream>>>(
-          h->d_act, hist_hess(h) ? h->d_act_h : nullptr, h->d_act_count, h->d_act_sub, h->d_selected, ds->n, h->n_blocks);
+          h->d_act, hist_hess(h) ? h->d_act_h : nullptr, h->d_act_count, h->d_selected, ds->n, h->n_blocks);
       h->launches_total++;
       YGG_RETURN_IF_ERROR(check_launch("k_compact_root"));
     }
@@ -867,43 +792,26 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
       ProfScope ps_level(h, kHistLevelNames[l & 15]);
       // zero the histogram planes (not the stats tail, which holds this level's node statistics)
       YGG_RETURN_IF_ERROR(zero_planes(h, lb));
-      if (h->hist_mode[l] == kHistRootSum) {
+      if (h->hist[l].mode == kHistRootSum) {
         // the root's counts do not depend on the gradients: reuse the precomputed (per-rank) ones,
         // d_root_cnt is [W * f_chunk][256] so that every chunk's count plane is one row of a 2-D copy
         const size_t row = static_cast<size_t>(lb.f_chunk) * kMaxBins * sizeof(uint32_t);
         YGG_CUDA(cudaMemcpy2DAsync(lb.cnt, lb.chunk_u64 * sizeof(unsigned long long), h->d_root_cnt, row, row, lb.W,
                                    cudaMemcpyDeviceToDevice, h->stream));
       }
-      if (h->hist2_FL[l] > 0) {
-        YGG_RETURN_IF_ERROR(ensure_bins4(h->ds));
-        Hist2Params hp{};
-        hp.bins4 = ds->d_bins4; hp.n_pad = ds->n_pad; hp.n = ds->n; hp.q24 = h->d_q24; hp.act = h->d_act;
-        hp.act_count = h->d_act_count; hp.act_sub = h->d_act_sub; hp.n_blocks = h->n_blocks;
-        hp.f_begin = h->hist_f_begin; hp.f_count = hist_f_count;
-        hp.g_begin = h->hist_f_begin / 4; hp.n_groups = (h->hist_f_end + 3) / 4 - hp.g_begin;
-        hp.S = h->hist_S[l]; hp.T = h->hist2_T[l]; hp.chunk_blocks = h->hist_chunk[l];
-        hp.level = l; hp.levels = h->d_levels;
-        hp.hist_sum = lb.sum; hp.hist_cnt = lb.cnt;
-        hp.f_chunk = lb.f_chunk; hp.chunk_stride = static_cast<long long>(lb.chunk_u64);
-        YGG_RETURN_IF_ERROR(launch_hist2(h, hp, h->hist2_FL[l], l == 0, h->hist_grid[l]));
-      } else {
+      const HistLevel& hl = h->hist[l];
       HistParams hp{};
       hp.bins = ds->d_bins; hp.n_pad = ds->n_pad; hp.act = h->d_act; hp.act_h = h->d_act_h; hp.q24 = h->d_q24;
       hp.act_count = h->d_act_count; hp.n_blocks = h->n_blocks;
-      hp.f_begin = h->hist_f_begin; hp.f_count = hist_f_count; hp.G = h->hist_G[l]; hp.S = h->hist_S[l];
-      hp.chunk_blocks = h->hist_chunk[l];
+      hp.f_begin = h->hist_f_begin; hp.f_count = hist_f_count; hp.G = hl.G; hp.S = hl.S;
+      hp.chunk_blocks = hl.chunk_blocks;
       hp.level = l; hp.levels = h->d_levels;
       hp.hist_sum = lb.sum; hp.hist_cnt = lb.cnt; hp.hist_hsum = lb.hsum;
       hp.f_chunk = lb.f_chunk; hp.chunk_stride = static_cast<long long>(lb.chunk_u64);
-      if (h->hist_passes[l] > 1) {
-        const int window = h->hist_S[l] - 1;
-        for (int pass = 0; pass < h->hist_passes[l]; pass++) {
-          hp.level = l | ((pass * window) << 8) | (window << 20);   // slot window of this pass (HistParams.level)
-          YGG_RETURN_IF_ERROR(launch_hist(h, hp, h->hist_mode[l], h->hist_grid[l], h->hist_smem[l], true));
-        }
-      } else {
-        YGG_RETURN_IF_ERROR(launch_hist(h, hp, h->hist_mode[l], h->hist_grid[l], h->hist_smem[l]));
-      }
+      const int window = hl.S - 1;
+      for (int pass = 0; pass < hl.passes; pass++) {
+        if (hl.passes > 1) hp.level = l | ((pass * window) << 8) | (window << 20);   // slot window of this pass (HistParams.level)
+        YGG_RETURN_IF_ERROR(launch_hist(h, hp, hl));
       }
     }
     if (h->capture_hist)   // this rank's own planes, before any collective
@@ -994,7 +902,7 @@ int grow_tree(ygg_gbt* h, NodeRec* nodes) {
       pp.n = ds->n; pp.level = l; pp.levels = h->d_levels; pp.nodes = nodes; pp.bins = ds->d_bins;
       pp.n_pad = ds->n_pad; pp.node_of_row = h->d_node_of_row; pp.n_blocks = h->n_blocks;
       pp.q24 = h->d_q24; pp.hq24 = hist_hess(h) ? h->d_hq24 : nullptr;
-      pp.act = h->d_act; pp.act_h = h->d_act_h; pp.act_count = h->d_act_count; pp.act_sub = h->d_act_sub;
+      pp.act = h->d_act; pp.act_h = h->d_act_h; pp.act_count = h->d_act_count;
       pp.selected = sampling(h) ? h->d_selected : nullptr;
       pp.g = h->cur_g; pp.h = has_h(h) ? h->cur_h : nullptr; pp.st = h->d_st; pp.stats = lbn.stats;
       // Child-statistic accumulators in shared memory: with few children (top levels) every warp
@@ -1798,7 +1706,6 @@ int ygg_dataset_destroy(ygg_dataset* ds) {
   if (!ds) return YGG_OK;
   cudaSetDevice(ds->device);
   dev_free(ds->d_bins);
-  dev_free(ds->d_bins4);
   dev_free(ds->d_num_bins);
   dev_free(ds->d_na_bin);
   dev_free(ds->d_feature_type);
@@ -1872,6 +1779,7 @@ int ygg_gbt_create(ygg_gbt** out, ygg_dataset* ds, const ygg_gbt_config* cfg) {
   YGG_CUDA(cudaSetDevice(ds->device));
   auto* h = new ygg_gbt();
   h->ds = ds;
+  h->device = ds->device;
   h->cfg = *cfg;
   // any failure below releases everything the handle already owns (stream, device buffers: the pool would otherwise
   // keep them for the life of the process and a retry with smaller settings could fail again)
@@ -1932,7 +1840,6 @@ static int init_handle(ygg_gbt* h) {
   YGG_RETURN_IF_ERROR(dev_alloc(&h->d_q24, n_pad));
   YGG_RETURN_IF_ERROR(dev_alloc(&h->d_act, n_pad));
   YGG_RETURN_IF_ERROR(dev_alloc(&h->d_act_count, h->n_blocks));
-  YGG_RETURN_IF_ERROR(dev_alloc(&h->d_act_sub, static_cast<size_t>(h->n_blocks) * kSubPerBlock));
   if (hist_hess(h)) {
     YGG_RETURN_IF_ERROR(dev_alloc(&h->d_hq24, n_pad));
     YGG_RETURN_IF_ERROR(dev_alloc(&h->d_act_h, n_pad));
@@ -1963,12 +1870,12 @@ static int init_handle(ygg_gbt* h) {
 
 int ygg_gbt_destroy(ygg_gbt* h) {
   if (!h) return YGG_OK;
-  cudaSetDevice(h->ds->device);
+  cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
   collect_profile(h);
   dev_free(h->d_label_u8); dev_free(h->d_label_f32); dev_free(h->d_pred); dev_free(h->d_g); dev_free(h->d_h);
   dev_free(h->d_q24); dev_free(h->d_hq24); dev_free(h->d_act); dev_free(h->d_act_h);
-  dev_free(h->d_act_count); dev_free(h->d_act_sub); dev_free(h->d_root_cnt); dev_free(h->d_node_of_row); dev_free(h->d_st); dev_free(h->d_levels);
+  dev_free(h->d_act_count); dev_free(h->d_root_cnt); dev_free(h->d_node_of_row); dev_free(h->d_st); dev_free(h->d_levels);
   for (int i = 0; i < 2; i++) {
     dev_free(h->d_fam[i]); dev_free(h->d_slot_node[i]); dev_free(h->d_hist_sum[i]); dev_free(h->d_hist_cnt[i]);
     dev_free(h->d_hist_hsum[i]);

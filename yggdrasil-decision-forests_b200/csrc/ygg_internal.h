@@ -12,7 +12,6 @@ struct ygg_dataset {
   int64_t n = 0, n_pad = 0;
   int F = 0;
   uint8_t* d_bins = nullptr;
-  uint32_t* d_bins4 = nullptr;   // interleaved copy [ceil(F/4)][n_pad] for k_hist2 (built on first use, ygg_hist2.cuh)
   int32_t* d_num_bins = nullptr;
   int32_t* d_na_bin = nullptr;
   int32_t* d_feature_type = nullptr;

@@ -18,7 +18,6 @@
 
 #include "ygg_device.cuh"
 #include "ygg_hist.cuh"
-#include "ygg_hist2.cuh"
 
 namespace ygg {
 
@@ -294,7 +293,7 @@ __global__ void __launch_bounds__(256) k_quantize(QuantParams p) {
 // hold the sampled rows only.  k_quantize wrote them dense; one CTA per 8192-row block compacts them in place, in row
 // order (entries go to registers first, so reading and writing the same list is safe).
 constexpr int kCompactThreads = 512;
-__global__ void __launch_bounds__(kCompactThreads) k_compact_root(uint2* act, uint32_t* act_h, int32_t* act_count, int32_t* act_sub,
+__global__ void __launch_bounds__(kCompactThreads) k_compact_root(uint2* act, uint32_t* act_h, int32_t* act_count,
                                                                   const uint8_t* __restrict__ selected, int64_t n, int n_blocks) {
   constexpr int R = kBlockRows / kCompactThreads;   // 16 consecutive rows per thread
   __shared__ int s_warp_tot[kCompactThreads / 32];
@@ -326,8 +325,6 @@ __global__ void __launch_bounds__(kCompactThreads) k_compact_root(uint2* act, ui
       if (w < warp) offset += t;
       total += t;
     }
-    // sub-tile boundaries (1024 rows = 64 threads)
-    if ((threadIdx.x & (kSubRows / R - 1)) == 0) act_sub[static_cast<int64_t>(blk) * kSubPerBlock + threadIdx.x / (kSubRows / R)] = offset;
     if (threadIdx.x == 0) act_count[blk] = total;
     __syncthreads();
 #pragma unroll
@@ -1030,7 +1027,6 @@ struct PartParams {
   uint2* act;
   uint32_t* act_h;
   int32_t* act_count;
-  int32_t* act_sub;           // [n_blocks][8] active rows before each 1024-row sub-tile of the block (k_hist2)
   const uint8_t* selected;    // stochastic gradient boosting: rows outside the sample are routed but not counted (null: all rows)
   const float* g;
   const float* h;   // null: h == 1
@@ -1123,7 +1119,6 @@ __global__ void __launch_bounds__(kPartThreads, 2) k_partition(PartParams p) {
     int written = 0;  // active rows of this block compacted so far
     if (nl.num_nodes == 0) {
       if (threadIdx.x == 0) p.act_count[blk] = 0;
-      if (threadIdx.x < kSubPerBlock) p.act_sub[static_cast<int64_t>(blk) * kSubPerBlock + threadIdx.x] = 0;
       continue;
     }
 #pragma unroll 1
@@ -1237,9 +1232,6 @@ __global__ void __launch_bounds__(kPartThreads, 2) k_partition(PartParams p) {
         total += t;
       }
       __syncthreads();
-      // sub-tile boundaries: the thread that owns the first row of a 1024-row sub-tile knows how many active rows precede it
-      if ((threadIdx.x & (kSubRows / kPartRows - 1)) == 0)
-        p.act_sub[static_cast<int64_t>(blk) * kSubPerBlock + pass * (kPartPassRows / kSubRows) + threadIdx.x / (kSubRows / kPartRows)] = offset;
       written += total;
       if (mine > 0) {
 #pragma unroll
